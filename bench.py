@@ -4,6 +4,8 @@
     python bench.py --gpus N --steps K --warmup W            # our arm (one process per GPU under torchrun for N>1)
     python bench.py --impl reference --steps K --warmup W    # the UNMODIFIED reference's PyTorch CPU forward on the host
     python bench.py --config {c,e,2x_fp32}                   # c (default) = the metric's config; e / 2x_fp32 = configs 4 / 5
+    python bench.py --dump-outputs DIR                       # also write the last timed step's detections / indices (.npy) to
+                                                             # DIR: same arguments, same inputs, so two builds can be compared
 
 One JSON line on stdout (rank 0).
   value         whole-job images/s, inputs resident in HBM, CUDA events, max over ranks
@@ -178,6 +180,26 @@ def check_parity(cfg, st, mode, base, dets, inds, n_check):
         min(n_check, n_base, B), max(B - n_base, 0))
 
 
+DUMP_BYTES = 64_000_000
+
+
+def dump_outputs(path, arrays):
+    """Writes what one timed step returned as <path>/<name>.npy, so that two builds can be compared output for output: float32
+    arrays as they are, integer ones as float64 (exact).  The arrays share the batch axis; if together they exceed 64 MB, the
+    same fixed, seeded sample of images is kept from each and its batch indices are written as sample.npy."""
+    arrays = {k: v if v.dtype == np.float32 else v.astype(np.float64) for k, v in arrays.items()}
+    B = next(iter(arrays.values())).shape[0]
+    per_image = sum(v.nbytes for v in arrays.values()) // B
+    if per_image * B > DUMP_BYTES:
+        n = (DUMP_BYTES - 4096 * (len(arrays) + 1)) // (per_image + 8)          # room for the .npy headers and sample.npy
+        keep = np.sort(np.random.default_rng(0).choice(B, n, replace=False))
+        arrays = {k: v[keep] for k, v in arrays.items()}
+        arrays["sample"] = keep.astype(np.float64)
+    os.makedirs(path, exist_ok=True)
+    for k, v in arrays.items():
+        np.save(os.path.join(path, k + ".npy"), np.ascontiguousarray(v))
+
+
 def run_ours(args):
     import torch
     import torch.distributed as dist
@@ -260,6 +282,8 @@ def run_ours(args):
 
     # ---- parity of what was just timed (outside the timed region): every rank checks its own images --------------------
     dev_dets, dev_inds = out["dets"].cpu().numpy(), out["inds"].cpu().numpy()
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, {"dets": dev_dets, "inds": dev_inds})
     n_check = args.parity_images if world == 1 else min(args.parity_images, 4)
     p_ok, p_msg = check_parity(cfg, st, args.offset_mode, base, dev_dets, dev_inds, n_check)
     parity_ok = all_ok(p_ok)
@@ -535,7 +559,11 @@ def main():
     ap.add_argument("--no-cpu", action="store_true", help="skip the cpu_baseline leg (profiling runs only)")
     ap.add_argument("--no-port", action="store_true", help="cpu_baseline: skip the numpy-port number beside the reference's")
     ap.add_argument("--dump-ops", default="", help="write the per-op device times (JSON) to this file")
+    ap.add_argument("--dump-outputs", default="", metavar="DIR",
+                    help="write rank 0's detections and indices of the last timed step to DIR/<name>.npy (float32 / float64)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     if args.config == "2x_fp32":
         from tools import bench_f32_config5
         return bench_f32_config5.main(args)

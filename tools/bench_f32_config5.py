@@ -128,6 +128,8 @@ def run_ours(args, C):
     barrier()
     ms = maxr(e0.elapsed_time(e1))
     value = world * B * args.steps / (ms / 1e3)
+    if args.dump_outputs and rank == 0:
+        bench.dump_outputs(args.dump_outputs, {"dets": static["dets"].cpu().numpy(), "inds": static["inds"].cpu().numpy()})
     # end to end: fp32 NCHW images from pinned host memory each step, detections back to the host
     dets_h = torch.empty((B, 100, 6), dtype=torch.float32).pin_memory()
     n_e2e = max(4, min(args.steps, 10))
