@@ -113,6 +113,10 @@ EXPORTS = {
     "cdn_engine_run_host_u8": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int, C.c_void_p, C.c_void_p]),
     "cdn_warp_affine_u8": (C.c_int, [C.c_void_p, C.c_int, C.c_int, C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_void_p]),
     "cdn_ctdet_group_by_class": (C.c_int, [C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p]),
+    "cdn_soft_nms": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_float, C.c_float, C.c_float, C.c_int, C.c_void_p,
+                               C.c_void_p]),
+    "cdn_ctdet_merge": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_int, C.c_void_p, C.c_int, C.c_int,
+                                  C.c_void_p, C.c_void_p, C.c_void_p]),
     "cdn_quantize_f32_i8": (C.c_int, [C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_int, C.c_double, C.c_double, C.c_void_p, C.c_int, C.c_void_p]),
     "cdn_maxpool3s2_i8": (C.c_int, [C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_int, C.c_void_p, C.c_void_p]),
     "cdn_engine_submit_host": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int, C.c_void_p, C.c_void_p, C.c_int]),

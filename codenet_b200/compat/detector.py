@@ -3,7 +3,8 @@
 `CtdetDetector(opt)` builds the network, quantises it, loads the checkpoint (`opt.load_model`, reference key space),
 freezes the activation ranges and runs forward + decode through the compiled int8 engine.  `run()` returns the same
 dict as the reference (`results` keyed by 1-based class id and the stage timers test.py prints, test.py:76-79).
-Only what differs from the reference lives here: engine construction, process / process_u8, the device-side box transform.
+Only what differs from the reference lives here: engine construction, process / process_u8, the device-side box transform,
+and run()'s multi-scale path (all test scales of an image in one engine batch, merge_outputs on the device: cdn_ctdet_merge).
 pre_process, merge_outputs and run keep the reference's contract (same inputs, outputs and timer keys) in this package's own
 decomposition (input_geometry / _Stages / group_by_class); INTEGRATION.md section 2 shows the patch for users who keep the reference's BaseDetector.
 """
@@ -370,37 +371,139 @@ class CtdetDetector:
             return cv2.imread(src), None
         return src['image'][0].numpy(), src
 
-    def run(self, image_or_path_or_tensor, meta=None):
-        clock = _Stages()
-        image, prepared = self._image_of(image_or_path_or_tensor)
-        clock.lap("load")
-        per_scale = []
+    def _slots_u8(self, image, scales, ih, iw):
+        """The network images of `scales` of one uint8 HWC frame as one uint8 CUDA batch [slots, ih, iw, 3] (scale-major, the
+        mirror after its image): an input-sized frame at scale 1 is copied as it is (resize and warpAffine are the identity),
+        any other frame goes through the host cv2.resize of pre_process (scale 1: none) and cdn_warp_affine_u8 writes it,
+        mirror included, into its slots.  Returns (batch, metas)."""
+        import ctypes as C
+        import cv2
+        from .. import _lib
+        n = 2 if self.opt.flip_test else 1
+        dev = self.opt.device
+        dst = torch.empty((n * len(scales), ih, iw, 3), dtype=torch.uint8, device=dev)
+        metas = []
+        with torch.cuda.device(dev):
+            st = C.c_void_p(torch.cuda.current_stream(dev).cuda_stream)
+            for k, scale in enumerate(scales):
+                (sh, sw), _, c, s = self.input_geometry(image.shape[0], image.shape[1], scale)
+                metas.append(self._meta(c, s, ih, iw))
+                if self._is_identity_input(image, scale):
+                    dst[k].copy_(torch.from_numpy(np.ascontiguousarray(image)))
+                    continue
+                src = image if scale == 1 else cv2.resize(image, (sw, sh))
+                src = torch.from_numpy(np.ascontiguousarray(src)).to(dev)
+                M = np.ascontiguousarray(get_affine_transform(c, s, 0, [iw, ih]), dtype=np.float64)
+                _lib.check(_lib.load().cdn_warp_affine_u8(C.c_void_p(src.data_ptr()), src.shape[0], src.shape[1], C.c_void_p(M.ctypes.data),
+                                                          C.c_void_p(dst[n * k].data_ptr()), ih, iw, n - 1, st))
+        return dst, metas
+
+    def _merge_on_device(self, dets, metas, clock):
+        """post_process of every scale + merge_outputs for the detections [S, K, 6] of one image's S test scales: one
+        post-affine with the per-scale transforms, one grouping, one cdn_ctdet_merge and one copy back.  When S x K exceeds the
+        device merge's segment limit the per-scale post_process and the host merge_outputs take over."""
+        import ctypes as C
+        from .. import _lib
+        S, K, nc = dets.shape[0], dets.shape[1], self.num_classes
+        if S * K > MERGE_MAX_ROWS:
+            per_scale = [self.post_process(dets[i:i + 1], metas[i], scale) for i, scale in enumerate(self.scales)]
+            clock.lap("post")
+            results = self.merge_outputs(per_scale)
+            clock.lap("merge")
+            return results
+        d = dets.detach().to(self.opt.device, torch.float32).contiguous().clone()
+        t = np.ascontiguousarray(np.stack([get_affine_transform(m['c'], m['s'], 0, (m['out_width'], m['out_height']), inv=1).reshape(6)
+                                           for m in metas]), dtype=np.float64)
+        g = torch.empty_like(d)
+        counts = torch.empty((S, nc), dtype=torch.int32, device=d.device)
+        buf = torch.empty(S * K * 5 + nc, dtype=torch.float32, device=d.device)     # rows, then the class counts (int32)
+        divisors = np.ascontiguousarray(self.scales, dtype=np.float32)
+        with torch.cuda.device(d.device):
+            st = C.c_void_p(torch.cuda.current_stream(d.device).cuda_stream)
+            L = _lib.load()
+            _lib.check(L.cdn_ctdet_post_affine(C.c_void_p(d.data_ptr()), S, K, C.c_void_p(t.ctypes.data), st))
+            _lib.check(L.cdn_ctdet_group_by_class(C.c_void_p(d.data_ptr()), S, K, nc, C.c_void_p(g.data_ptr()),
+                                                  C.c_void_p(counts.data_ptr()), st))
+            clock.lap("post")
+            _lib.check(L.cdn_ctdet_merge(C.c_void_p(g.data_ptr()), C.c_void_p(counts.data_ptr()), 1, S, K, nc,
+                                         C.c_void_p(divisors.ctypes.data), int(bool(self.opt.nms)), self.max_per_image,
+                                         C.c_void_p(buf.data_ptr()), C.c_void_p(buf[S * K * 5:].data_ptr()), st))
+        host = buf.cpu().numpy()
+        rows, cnt = host[:S * K * 5].reshape(-1, 5), host[S * K * 5:].view(np.int32)
+        ends = np.cumsum(cnt)
+        results = {j + 1: rows[ends[j] - cnt[j]:ends[j]] for j in range(nc)}
+        clock.lap("merge")
+        return results
+
+    def _run_float(self, image, prepared, clock):
+        """run() of the unquantised model: one network call per scale as before (its uint8 normalisation runs in torch fp32,
+        which is not what pre_process computes at scales other than 1), then the device merge."""
+        dets, metas = [], []
         for scale in self.scales:
             if prepared is not None:
                 images = prepared['images'][scale][0]
                 meta = {k: (v.numpy()[0] if torch.is_tensor(v) else v) for k, v in prepared['meta'][scale].items()}
-                fn = self.process
-            elif self._is_identity_input(image, scale):
-                # ship the uint8 image as it is; the stem kernel normalises through the 3 x 256 table
-                h, w = image.shape[:2]
-                images = torch.from_numpy(np.ascontiguousarray(image[None]))
-                meta = self._meta(np.array([w / 2., h / 2.], np.float32), float(max(h, w)), h, w)
-                fn = self.process_u8
             elif scale == 1 and image.dtype == np.uint8 and image.ndim == 3 and getattr(self.opt, "device_pre_process", True):
-                images, meta = self.pre_process_device(image, scale, meta)           # warpAffine (+ mirror) on the device
-                fn = self.process
+                images, meta = self.pre_process_device(image, scale)
             else:
-                images, meta = self.pre_process(image, scale, meta)
-                fn = self.process
+                images, meta = self.pre_process(image, scale)
             images = images.to(self.opt.device)
             torch.cuda.synchronize()
             clock.lap("pre")
-            output, dets, t_forward = fn(images, return_time=True)
+            _, d, t_forward = self.process(images, return_time=True)
             torch.cuda.synchronize()
             clock.lap("net", t_forward)
             clock.lap("dec")
-            per_scale.append(self.post_process(dets, meta, scale))
-            clock.lap("post")
-        results = self.merge_outputs(per_scale)
-        clock.lap("merge")
-        return clock.result(results)
+            dets.append(d[:1])
+            metas.append(meta)
+        return self._merge_on_device(torch.cat(dets, 0), metas, clock)
+
+    def run(self, image_or_path_or_tensor, meta=None):
+        """All test scales of the image that share one network input size (all of them with fix_res) go through the engine as
+        one batch, scale-major with every mirror right after its image; then one post-affine, grouping and merge on the device
+        for all scales and one copy back (merge_outputs on the host only when scales x K exceeds the device merge's limit)."""
+        clock = _Stages()
+        image, prepared = self._image_of(image_or_path_or_tensor)
+        clock.lap("load")
+        if self.float_model:
+            return clock.result(self._run_float(image, prepared, clock))
+        if prepared is not None:
+            sizes = [tuple(int(v) for v in prepared['images'][scale][0].shape[-2:]) for scale in self.scales]
+        else:
+            sizes = [self.input_geometry(image.shape[0], image.shape[1], scale)[1] for scale in self.scales]
+        u8 = (prepared is None and image.dtype == np.uint8 and image.ndim == 3 and image.shape[2] == 3 and
+              (getattr(self.opt, "device_pre_process", True) or all(self._is_identity_input(image, s) for s in self.scales)))
+        dets, metas = [None] * len(self.scales), [None] * len(self.scales)
+        for (ih, iw), idx in plan_scale_batches(sizes):
+            scales = [self.scales[i] for i in idx]
+            if prepared is not None:
+                images = torch.cat([prepared['images'][scale][0] for scale in scales], 0)
+                ms = [{k: (v.numpy()[0] if torch.is_tensor(v) else v) for k, v in prepared['meta'][scale].items()} for scale in scales]
+            elif u8:
+                images, ms = self._slots_u8(image, scales, ih, iw)
+            else:
+                pre = [self.pre_process(image, scale) for scale in scales]
+                images, ms = torch.cat([p[0] for p in pre], 0), [p[1] for p in pre]
+            images = images.to(self.opt.device)
+            torch.cuda.synchronize()
+            clock.lap("pre")
+            _, d, t_forward = self.process(images, return_time=True)
+            torch.cuda.synchronize()
+            clock.lap("net", t_forward)
+            clock.lap("dec")
+            for k, i in enumerate(idx):
+                dets[i], metas[i] = d[k:k + 1], ms[k]
+        return clock.result(self._merge_on_device(torch.cat(dets, 0), metas, clock))
+
+
+MERGE_MAX_ROWS = 1024          # CDN_SOFT_NMS_MAX_LEN: test scales x K rows per image that cdn_ctdet_merge takes
+
+
+def plan_scale_batches(sizes):
+    """Network input size (h, w) of every test scale -> [((h, w), [scale indices])], one batch per distinct size in the order
+    of first appearance, scales in their order inside a batch.  The engine batch is scale-major: slot k (or slots 2k, 2k+1
+    with the --flip_test mirror right after its image, the order process() pairs them in) holds the k-th scale of the list."""
+    groups = {}
+    for i, hw in enumerate(sizes):
+        groups.setdefault(tuple(int(v) for v in hw), []).append(i)
+    return list(groups.items())

@@ -1,12 +1,13 @@
 """Host-side mirror of the reference's `soft_nms` (lib/models/external/nms.pyx:77-170), used by
-`CtdetDetector.merge_outputs` for multi-scale testing and `--nms` (lib/detectors/ctdet.py:59-74).
+`CtdetDetector.merge_outputs` for multi-scale testing and `--nms` (lib/detectors/ctdet.py:59-74), and its device form
+`soft_nms_device` (cdn_soft_nms, many segments in one launch), which CtdetDetector.run() reaches through cdn_ctdet_merge.
 
-The reference runs this on the CPU as well (compiled Cython); it is not part of the accelerated path.  The restatement
-keeps the reference's in-place semantics and its single-precision arithmetic (`cdef float` temporaries; `np.exp` evaluated
+The reference runs this on the CPU (compiled Cython).  The restatement keeps the reference's in-place semantics and its single-precision arithmetic (`cdef float` temporaries; `np.exp` evaluated
 in double and rounded to float), so results are bit-identical to the compiled reference (tests/golden/soft_nms_kat.npz):
 
   * `boxes` [N, 5] float32 (x1, y1, x2, y2, score) is modified IN PLACE: selection-sorts by score, decays the scores of
-    overlapping boxes, and swaps boxes whose score falls below `threshold` to the tail;
+    overlapping boxes, and overwrites a box whose score falls below `threshold` with a COPY of the last box (the discarded
+    box is lost; rows past the final N keep stale copies with their scores from before that pass);
   * the outer loop runs over the ORIGINAL N (Cython evaluates `range(N)` once) while the inner loops use the shrinking N;
   * returns `list(range(N_final))`, which `merge_outputs` ignores -- it keeps every row of the modified array.
 """
@@ -57,3 +58,29 @@ def soft_nms(boxes, sigma=0.5, Nt=0.3, threshold=0.001, method=0):
                         pos -= 1
             pos += 1
     return list(range(N))
+
+
+def soft_nms_device(boxes, seg_off, sigma=0.5, Nt=0.3, threshold=0.001, method=0):
+    """soft_nms on the device over independent segments: `boxes` CUDA float32 [rows, 5] (contiguous), segment g = rows
+    seg_off[g] .. seg_off[g+1] (host sequence of n_seg + 1 non-decreasing offsets), each modified in place exactly as
+    soft_nms(boxes[seg], sigma, Nt, threshold, method) modifies its array.  Returns the keep counts (len of soft_nms's
+    result) as an int32 CUDA tensor [n_seg]; asynchronous on the current stream.  A segment longer than
+    CDN_SOFT_NMS_MAX_LEN (1024) rows raises CdnError before anything is launched."""
+    import ctypes as C
+    import torch
+    from .. import _lib
+    if not (torch.is_tensor(boxes) and boxes.is_cuda and boxes.dtype == torch.float32 and boxes.dim() == 2 and boxes.shape[1] == 5
+            and boxes.is_contiguous()):
+        raise ValueError("soft_nms_device takes a contiguous CUDA float32 [rows, 5] tensor")
+    off = np.asarray(seg_off, dtype=np.int64).reshape(-1)
+    if off.size < 1 or off[0] < 0 or off[-1] > boxes.shape[0] or (np.diff(off) < 0).any():
+        raise ValueError("seg_off must be non-decreasing offsets into the rows of boxes")
+    n_seg = off.size - 1
+    max_len = int(np.diff(off).max()) if n_seg else 0
+    keep = torch.empty(n_seg, dtype=torch.int32, device=boxes.device)
+    d_off = torch.from_numpy(off.astype(np.int32)).to(boxes.device)
+    with torch.cuda.device(boxes.device):
+        _lib.check(_lib.load().cdn_soft_nms(C.c_void_p(boxes.data_ptr()), C.c_void_p(d_off.data_ptr()), n_seg, max_len, float(sigma),
+                                            float(Nt), float(threshold), int(method), C.c_void_p(keep.data_ptr()),
+                                            C.c_void_p(torch.cuda.current_stream(boxes.device).cuda_stream)))
+    return keep

@@ -18,6 +18,9 @@
  *   cdn_dw3x3_i8                  <- QuantBnConv2d.forward for depthwise 3x3 convs (same lines) + QuantAct
  *   cdn_stem_f32_i8               <- layer0 = QuantBnConv2d(8 bit) + ReLU + QuantAct [+ MaxPool], quantize_model.py:26-35
  *   cdn_ctdet_decode              <- ctdet_decode, lib/models/decode.py:474-505 (_nms :10-16, _topk :110-126)
+ *   cdn_ctdet_merge               <- CtdetDetector.merge_outputs, lib/detectors/ctdet.py:59-74 (with post_process's division by the
+ *                                    scale, base_detector.py post_process)
+ *   cdn_soft_nms                  <- soft_nms, lib/models/external/nms.pyx:77-170
  *   cdn_engine_*                  <- PoseShuffleNetV2.forward (shufflenetv2_dcn.py:314-330) as rewritten by
  *                                    quantize_shufflenetv2_dcn (quantize_model.py:7-82) + CtdetDetector.process
  *                                    (lib/detectors/ctdet.py:29-46)
@@ -129,6 +132,35 @@ int cdn_warp_affine_u8(const uint8_t* d_src, int H, int W, const double* M6, uin
                        cdn_stream_t stream);
 int cdn_ctdet_group_by_class(const float* d_dets, int batch, int K, int num_classes, float* d_out, int32_t* d_counts,
                              cdn_stream_t stream);
+
+/* ---- multi-scale merge and soft-NMS (lib/detectors/ctdet.py:59-74, lib/models/external/nms.pyx:77-170) ---------------
+ * cdn_soft_nms: the reference's soft_nms on n_seg independent segments of d_boxes [rows][5] (x1, y1, x2, y2, score), segment g =
+ * rows [d_seg_off[g], d_seg_off[g+1]) (device int32, non-overlapping), each modified IN PLACE exactly as compat.soft_nms
+ * modifies its array: the outer loop over the original length, the first maximum with row i winning ties, a discarded row
+ * overwritten by a copy of row N-1, rows past the final N holding stale copies with their scores from before the pass.
+ * d_keep[g] = the final N (what len(soft_nms(...)) returns).  method 0 hard, 1 linear, 2 gaussian.  Bit-identical to the mirror
+ * (float / double sequence of compat/nms.py:40-53, exp = CUDA's double exp rounded to float).  max_len is the caller's bound on
+ * the segment lengths; max_len > CDN_SOFT_NMS_MAX_LEN is CDN_ERR_INVALID before anything is launched, and a segment longer than
+ * max_len (or with a negative start or length) is left untouched with d_keep = -1.  Scores must not be NaN.  Asynchronous.
+ * cdn_ctdet_merge: CtdetDetector.merge_outputs (ctdet.py:59-74) for `batch` images with `scales` test scales each.  Inputs are
+ * the outputs of cdn_ctdet_post_affine + cdn_ctdet_group_by_class for batch * scales network images, image-major and
+ * scale-minor: d_grouped [batch*scales][K][6], d_counts [batch*scales][num_classes]; h_scales [scales] (host) the divisors of
+ * post_process (base_detector.py post_process: coordinates / scale as a float32 division).  Per image and class the rows of
+ * scale 0, 1, ... in grouped order (np.vstack order), coordinates divided by the scale; when scales > 1 or nms != 0 soft-NMS
+ * per class with Nt 0.5, method 2, sigma 0.5, threshold 0.001, every row kept, stale tail included; then, if more than
+ * max_per_image rows remain, only rows scoring >= the max_per_image-th largest score (np.partition) survive, in their order
+ * (ties at the cut can keep more).  Outputs: d_rows [batch][scales*K][5] rows grouped by class (only the first
+ * sum(d_class_counts[b]) rows of an image are written), d_class_counts [batch][num_classes].  Needs scales*K <=
+ * CDN_SOFT_NMS_MAX_LEN, scales <= CDN_MERGE_MAX_SCALES, num_classes <= CDN_MERGE_MAX_CLASSES (CDN_ERR_INVALID otherwise,
+ * checked on the host); one CTA per image keeps every intermediate in shared memory, so there is no workspace, no allocation
+ * and no synchronisation: the call only enqueues one kernel on `stream`. */
+#define CDN_SOFT_NMS_MAX_LEN 1024
+#define CDN_MERGE_MAX_SCALES 16
+#define CDN_MERGE_MAX_CLASSES 1024
+int cdn_soft_nms(float* d_boxes, const int32_t* d_seg_off, int n_seg, int max_len, float sigma, float Nt, float threshold, int method,
+                 int32_t* d_keep, cdn_stream_t stream);
+int cdn_ctdet_merge(const float* d_grouped, const int32_t* d_counts, int batch, int scales, int K, int num_classes,
+                    const float* h_scales, int nms, int max_per_image, float* d_rows, int32_t* d_class_counts, cdn_stream_t stream);
 
 /* ---- module-level helpers: QuantAct on a real-valued tensor, MaxPool on the int8 grid -----------------------------
  * What compat.QuantAct.forward (portable_quantizer/quant_modules.py:202-225, frozen range) runs when it is handed an fp32
