@@ -36,6 +36,12 @@ class PwDesc(C.Structure):
                 ("n_f32", C.c_int), ("Mf", C.POINTER(C.c_double)), ("bf", C.POINTER(C.c_double))]
 
 
+# cdn_warp_desc (include/codenet_b200.h): one output image of cdn_warp_affine_u8_batch
+WARP_DESC = np.dtype([("src_offset", np.int64), ("src_h", np.int32), ("src_w", np.int32), ("M", np.float64, (6,)),
+                      ("dst_slot", np.int32), ("mirror_slot", np.int32)])
+assert WARP_DESC.itemsize == 72
+WARP_DESC_PER_LAUNCH = 454         # CDN_WARP_DESC_PER_LAUNCH
+
 EXPORTS = {
     "cdn_last_error": (C.c_char_p, []),
     "cdn_version": (C.c_int, []),
@@ -112,6 +118,7 @@ EXPORTS = {
                                     C.c_void_p, C.c_void_p]),
     "cdn_engine_run_host_u8": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int, C.c_void_p, C.c_void_p]),
     "cdn_warp_affine_u8": (C.c_int, [C.c_void_p, C.c_int, C.c_int, C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_void_p]),
+    "cdn_warp_affine_u8_batch": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int, C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_void_p]),
     "cdn_ctdet_group_by_class": (C.c_int, [C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p]),
     "cdn_soft_nms": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_float, C.c_float, C.c_float, C.c_int, C.c_void_p,
                                C.c_void_p]),

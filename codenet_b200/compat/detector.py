@@ -4,7 +4,8 @@
 freezes the activation ranges and runs forward + decode through the compiled int8 engine.  `run()` returns the same
 dict as the reference (`results` keyed by 1-based class id and the stage timers test.py prints, test.py:76-79).
 Only what differs from the reference lives here: engine construction, process / process_u8, the device-side box transform,
-and run()'s multi-scale path (all test scales of an image in one engine batch, merge_outputs on the device: cdn_ctdet_merge).
+run()'s multi-scale path (all test scales of an image in one engine batch, merge_outputs on the device: cdn_ctdet_merge) and
+run_batch() (many raw frames per engine step, their warpAffine in one cdn_warp_affine_u8_batch launch per step).
 pre_process, merge_outputs and run keep the reference's contract (same inputs, outputs and timer keys) in this package's own
 decomposition (input_geometry / _Stages / group_by_class); INTEGRATION.md section 2 shows the patch for users who keep the reference's BaseDetector.
 """
@@ -288,40 +289,51 @@ class CtdetDetector:
             raise RuntimeError("codenet_b200 has no CPU execution path: process() needs CUDA images")
         if self.float_model:
             return self._process_float(images, return_time)
-        if images.dtype == torch.uint8:
-            B, H, W, _ = images.shape
-            x = images.contiguous()
-        else:
-            B, _, H, W = images.shape
-            x = images.contiguous().float()
-        dev = images.device.index if images.device.index is not None else torch.cuda.current_device()
+        x = images.contiguous() if images.dtype == torch.uint8 else images.contiguous().float()
+        marks = []
+
+        def mark():                                  # the network's outputs are complete: the forward time of run()'s "net"
+            torch.cuda.synchronize(images.device)
+            marks.append(time.time())
+        output, dets = self._forward(x, mark=mark)
+        return (output, dets, marks[0]) if return_time else (output, dets)
+
+    def _forward(self, x, out=None, maps=True, mark=None):
+        """process() of the quantised model without a synchronisation: enqueues the engine and the decode on the current stream
+        and returns (output, dets).  x: contiguous CUDA uint8 [B,H,W,3] or fp32 [B,3,H,W].  `out`: Engine.run's output
+        buffers, kept by the caller so that the engine replays one graph (at least B images each); `maps=False` leaves the head
+        maps out where the detections do not need them.  `mark()`, if given, is called once the network's outputs are
+        enqueued, before the host-side decode steps."""
+        B = x.shape[0]
+        H, W = (x.shape[1], x.shape[2]) if x.dtype == torch.uint8 else (x.shape[2], x.shape[3])
+        dev = x.device.index if x.device.index is not None else torch.cuda.current_device()
         eng = self._engine_for(H, W, B, dev)
         if not self.opt.flip_test:
             # forward + sigmoid + decode in one graph replay; `hm` comes back post-sigmoid like output['hm'].sigmoid_()
-            out = eng.run(x, maps=True, dets=True)
-            torch.cuda.synchronize(images.device)
-            forward_time = time.time()
-            output = {h: out[h] for h in self.opt.heads}
-            dets = out["dets"] if self.opt.reg_offset else ctdet_decode(out["hm"], out["wh"], reg=None, K=self.opt.K)
+            out = eng.run(x, maps=maps or not self.opt.reg_offset, dets=True, out=out)
+            if mark is not None:
+                mark()
+            output = {h: out[h][:B] for h in self.opt.heads if h in out}
+            dets = out["dets"][:B] if self.opt.reg_offset else ctdet_decode(out["hm"][:B], out["wh"][:B], reg=None, K=self.opt.K)
         else:
             # image + mirrored image: average hm and wh with the mirror flipped back (ctdet.py:35-38), on the device
             import ctypes as C
             from .. import _lib
-            out = eng.run(x, maps=True, dets=False)
-            output = {h: out[h] for h in self.opt.heads}
+            out = eng.run(x, maps=True, dets=False, out=out)
+            output = {h: out[h][:B] for h in self.opt.heads}
             pairs = B // 2
-            hm = torch.empty((pairs,) + tuple(out["hm"].shape[1:]), dtype=torch.float32, device=images.device)
-            wh = torch.empty((pairs,) + tuple(out["wh"].shape[1:]), dtype=torch.float32, device=images.device)
-            with torch.cuda.device(images.device):
+            hm = torch.empty((pairs,) + tuple(out["hm"].shape[1:]), dtype=torch.float32, device=x.device)
+            wh = torch.empty((pairs,) + tuple(out["wh"].shape[1:]), dtype=torch.float32, device=x.device)
+            with torch.cuda.device(x.device):
                 _lib.check(_lib.load().cdn_ctdet_flip_merge(
                     C.c_void_p(out["hm"].data_ptr()), C.c_void_p(out["wh"].data_ptr()), pairs, hm.shape[1], hm.shape[2], hm.shape[3],
                     C.c_void_p(hm.data_ptr()), C.c_void_p(wh.data_ptr()),
-                    C.c_void_p(torch.cuda.current_stream(images.device).cuda_stream)))
-            reg = out["reg"][0::2].contiguous() if self.opt.reg_offset else None     # the unflipped image of every pair
-            torch.cuda.synchronize(images.device)
-            forward_time = time.time()
+                    C.c_void_p(torch.cuda.current_stream(x.device).cuda_stream)))
+            reg = out["reg"][0:B:2].contiguous() if self.opt.reg_offset else None     # the unflipped image of every pair
+            if mark is not None:
+                mark()
             dets = ctdet_decode(hm, wh, reg=reg, cat_spec_wh=self.opt.cat_spec_wh, K=self.opt.K)
-        return (output, dets, forward_time) if return_time else (output, dets)
+        return output, dets
 
     def post_process(self, dets, meta, scale=1):
         """dets [1|B,K,6] in output-map coordinates -> {class: [n,5]} in image coordinates.  The affine runs on the device
@@ -371,67 +383,95 @@ class CtdetDetector:
             return cv2.imread(src), None
         return src['image'][0].numpy(), src
 
+    def _frame_layout(self, height, width, scales):
+        """[(source height, source width, forward matrix, meta)] of `scales` for an height x width frame: the source of a scale is
+        the image pre_process hands to cv2.warpAffine (the frame itself at scale 1, its cv2.resize otherwise)."""
+        layout = []
+        for scale in scales:
+            (sh, sw), (ih, iw), c, s = self.input_geometry(height, width, scale)
+            layout.append((sh, sw, get_affine_transform(c, s, 0, [iw, ih]), self._meta(c, s, ih, iw)))
+        return layout
+
+    def _pack_frame(self, image, layout, scales, pool, offsets, desc, slot0):
+        """Writes the source image of every scale of one uint8 HWC frame into the byte pool at `offsets` (the frame at scale 1,
+        pre_process's host cv2.resize otherwise: DESIGN.md section 9) and fills its warp descriptors: slot0 + k for scale k, or
+        slot0 + 2k with the --flip_test mirror in slot0 + 2k + 1."""
+        import cv2
+        n = 2 if self.opt.flip_test else 1
+        for k, ((sh, sw, M, _), scale, off) in enumerate(zip(layout, scales, offsets)):
+            src = image if scale == 1 else cv2.resize(image, (sw, sh))
+            pool[off:off + sh * sw * 3] = np.ascontiguousarray(src).reshape(-1)
+            slot = slot0 + n * k
+            desc[k] = (off, sh, sw, np.asarray(M, np.float64).reshape(6), slot, slot + 1 if n == 2 else -1)
+
+    def _warp(self, pool, desc, dst):
+        """cdn_warp_affine_u8_batch on the current stream: the descriptors `desc` (_lib.WARP_DESC) from the device byte pool into
+        the uint8 CUDA batch dst [slots, H, W, 3]."""
+        import ctypes as C
+        from .. import _lib
+        st = C.c_void_p(torch.cuda.current_stream(dst.device).cuda_stream)
+        _lib.check(_lib.load().cdn_warp_affine_u8_batch(C.c_void_p(pool.data_ptr()), C.c_void_p(desc.ctypes.data), len(desc),
+                                                         C.c_void_p(dst.data_ptr()), dst.shape[0], dst.shape[1], dst.shape[2], st))
+
     def _slots_u8(self, image, scales, ih, iw):
         """The network images of `scales` of one uint8 HWC frame as one uint8 CUDA batch [slots, ih, iw, 3] (scale-major, the
-        mirror after its image): an input-sized frame at scale 1 is copied as it is (resize and warpAffine are the identity),
-        any other frame goes through the host cv2.resize of pre_process (scale 1: none) and cdn_warp_affine_u8 writes it,
-        mirror included, into its slots.  Returns (batch, metas)."""
-        import ctypes as C
-        import cv2
-        from .. import _lib
+        mirror after its image): the frame and its host cv2.resize copies (scales other than 1) go to the device in one byte pool
+        and one cdn_warp_affine_u8_batch launch writes every slot, mirrors included.  Returns (batch, metas)."""
+        from .._lib import WARP_DESC
         n = 2 if self.opt.flip_test else 1
         dev = self.opt.device
+        layout = self._frame_layout(image.shape[0], image.shape[1], scales)
+        (_, offsets, nbytes), = plan_frame_steps([[sh * sw * 3 for sh, sw, _, _ in layout]], n * len(scales), 1)
+        pool = np.empty(nbytes, np.uint8)
+        desc = np.empty(len(scales), WARP_DESC)
+        self._pack_frame(image, layout, scales, pool, offsets[0], desc, 0)
         dst = torch.empty((n * len(scales), ih, iw, 3), dtype=torch.uint8, device=dev)
-        metas = []
         with torch.cuda.device(dev):
-            st = C.c_void_p(torch.cuda.current_stream(dev).cuda_stream)
-            for k, scale in enumerate(scales):
-                (sh, sw), _, c, s = self.input_geometry(image.shape[0], image.shape[1], scale)
-                metas.append(self._meta(c, s, ih, iw))
-                if self._is_identity_input(image, scale):
-                    dst[k].copy_(torch.from_numpy(np.ascontiguousarray(image)))
-                    continue
-                src = image if scale == 1 else cv2.resize(image, (sw, sh))
-                src = torch.from_numpy(np.ascontiguousarray(src)).to(dev)
-                M = np.ascontiguousarray(get_affine_transform(c, s, 0, [iw, ih]), dtype=np.float64)
-                _lib.check(_lib.load().cdn_warp_affine_u8(C.c_void_p(src.data_ptr()), src.shape[0], src.shape[1], C.c_void_p(M.ctypes.data),
-                                                          C.c_void_p(dst[n * k].data_ptr()), ih, iw, n - 1, st))
-        return dst, metas
+            self._warp(torch.from_numpy(pool).to(dev), desc, dst)
+        return dst, [m for _, _, _, m in layout]
 
     def _merge_on_device(self, dets, metas, clock):
-        """post_process of every scale + merge_outputs for the detections [S, K, 6] of one image's S test scales: one
-        post-affine with the per-scale transforms, one grouping, one cdn_ctdet_merge and one copy back.  When S x K exceeds the
-        device merge's segment limit the per-scale post_process and the host merge_outputs take over."""
+        """post_process of every scale + merge_outputs for the detections [F*S, K, 6] of F images' S test scales (image-major,
+        scale-minor; metas likewise): one post-affine with the per-slot transforms, one grouping, one cdn_ctdet_merge over the F
+        images and one copy back.  Returns the F results.  When S x K exceeds the device merge's segment limit the per-scale
+        post_process and the host merge_outputs take over, image by image."""
         import ctypes as C
         from .. import _lib
-        S, K, nc = dets.shape[0], dets.shape[1], self.num_classes
+        S, K, nc = len(self.scales), dets.shape[1], self.num_classes
+        F = dets.shape[0] // S
         if S * K > MERGE_MAX_ROWS:
-            per_scale = [self.post_process(dets[i:i + 1], metas[i], scale) for i, scale in enumerate(self.scales)]
-            clock.lap("post")
-            results = self.merge_outputs(per_scale)
-            clock.lap("merge")
+            results = []
+            for f in range(F):
+                per_scale = [self.post_process(dets[f * S + i:f * S + i + 1], metas[f * S + i], scale) for i, scale in enumerate(self.scales)]
+                clock.lap("post")
+                results.append(self.merge_outputs(per_scale))
+                clock.lap("merge")
             return results
         d = dets.detach().to(self.opt.device, torch.float32).contiguous().clone()
         t = np.ascontiguousarray(np.stack([get_affine_transform(m['c'], m['s'], 0, (m['out_width'], m['out_height']), inv=1).reshape(6)
                                            for m in metas]), dtype=np.float64)
         g = torch.empty_like(d)
-        counts = torch.empty((S, nc), dtype=torch.int32, device=d.device)
-        buf = torch.empty(S * K * 5 + nc, dtype=torch.float32, device=d.device)     # rows, then the class counts (int32)
+        counts = torch.empty((F * S, nc), dtype=torch.int32, device=d.device)
+        R = S * K * 5                                                               # merged rows of one image
+        buf = torch.empty(F * (R + nc), dtype=torch.float32, device=d.device)      # rows, then the class counts (int32)
         divisors = np.ascontiguousarray(self.scales, dtype=np.float32)
         with torch.cuda.device(d.device):
             st = C.c_void_p(torch.cuda.current_stream(d.device).cuda_stream)
             L = _lib.load()
-            _lib.check(L.cdn_ctdet_post_affine(C.c_void_p(d.data_ptr()), S, K, C.c_void_p(t.ctypes.data), st))
-            _lib.check(L.cdn_ctdet_group_by_class(C.c_void_p(d.data_ptr()), S, K, nc, C.c_void_p(g.data_ptr()),
+            _lib.check(L.cdn_ctdet_post_affine(C.c_void_p(d.data_ptr()), F * S, K, C.c_void_p(t.ctypes.data), st))
+            _lib.check(L.cdn_ctdet_group_by_class(C.c_void_p(d.data_ptr()), F * S, K, nc, C.c_void_p(g.data_ptr()),
                                                   C.c_void_p(counts.data_ptr()), st))
             clock.lap("post")
-            _lib.check(L.cdn_ctdet_merge(C.c_void_p(g.data_ptr()), C.c_void_p(counts.data_ptr()), 1, S, K, nc,
+            _lib.check(L.cdn_ctdet_merge(C.c_void_p(g.data_ptr()), C.c_void_p(counts.data_ptr()), F, S, K, nc,
                                          C.c_void_p(divisors.ctypes.data), int(bool(self.opt.nms)), self.max_per_image,
-                                         C.c_void_p(buf.data_ptr()), C.c_void_p(buf[S * K * 5:].data_ptr()), st))
+                                         C.c_void_p(buf.data_ptr()), C.c_void_p(buf[F * R:].data_ptr()), st))
         host = buf.cpu().numpy()
-        rows, cnt = host[:S * K * 5].reshape(-1, 5), host[S * K * 5:].view(np.int32)
-        ends = np.cumsum(cnt)
-        results = {j + 1: rows[ends[j] - cnt[j]:ends[j]] for j in range(nc)}
+        cnts = host[F * R:].view(np.int32).reshape(F, nc)
+        results = []
+        for f in range(F):
+            rows, cnt = host[f * R:(f + 1) * R].reshape(-1, 5), cnts[f]
+            ends = np.cumsum(cnt)
+            results.append({j + 1: rows[ends[j] - cnt[j]:ends[j]] for j in range(nc)})
         clock.lap("merge")
         return results
 
@@ -456,7 +496,7 @@ class CtdetDetector:
             clock.lap("dec")
             dets.append(d[:1])
             metas.append(meta)
-        return self._merge_on_device(torch.cat(dets, 0), metas, clock)
+        return self._merge_on_device(torch.cat(dets, 0), metas, clock)[0]
 
     def run(self, image_or_path_or_tensor, meta=None):
         """All test scales of the image that share one network input size (all of them with fix_res) go through the engine as
@@ -493,7 +533,127 @@ class CtdetDetector:
             clock.lap("dec")
             for k, i in enumerate(idx):
                 dets[i], metas[i] = d[k:k + 1], ms[k]
-        return clock.result(self._merge_on_device(torch.cat(dets, 0), metas, clock))
+        return clock.result(self._merge_on_device(torch.cat(dets, 0), metas, clock)[0])
+
+    def run_batch(self, frames):
+        """run() for many raw frames: frames is a list of uint8 HWC 3-channel arrays and/or image paths (cv2.imread).  Returns
+        one dict per frame in run()'s format; element i's results are run(frames[i])'s, and the stage timers are the call's
+        totals divided evenly across its frames (summed over frames they give the wall time).
+
+        Engine steps of max(opt.max_batch, slots of one frame) slots hold whole frames, frame-major, every frame's slots
+        scale-major with each --flip_test mirror right after its image (plan_frame_steps).  Per step the raw frames and their
+        host cv2.resize copies (scales other than 1) are packed into a pinned staging buffer, sent with one copy on a copy
+        stream, and one cdn_warp_affine_u8_batch launch writes every slot; then the engine, the flip merge and decode.  Two
+        staging buffers, kept on the detector, let the packing and copy of step n + 1 overlap the compute of step n.  After the
+        last step one post-affine, grouping, cdn_ctdet_merge over all frames and one copy back (_merge_on_device).
+        Needs fix_res (the engine is compiled for one input size; run() is the path for keep_res); prefetched dicts go through
+        run().  The unquantised model runs run() frame by frame."""
+        clock = _Stages()
+        images = self._batch_frames(frames)
+        if not images:
+            return []
+        if self.float_model:
+            return [self.run(image) for image in images]
+        clock.lap("load")
+        opt, dev = self.opt, self.opt.device
+        n = 2 if opt.flip_test else 1
+        S, F, ih, iw = len(self.scales), len(images), opt.input_h, opt.input_w
+        spf = n * S
+        layouts = [self._frame_layout(im.shape[0], im.shape[1], self.scales) for im in images]
+        metas = [m for layout in layouts for _, _, _, m in layout]
+        max_batch = getattr(opt, "max_batch", 1)
+        steps = plan_frame_steps([[sh * sw * 3 for sh, sw, _, _ in layout] for layout in layouts], spf, max_batch)
+        step_slots = max(int(max_batch), spf)
+        from .._lib import WARP_DESC
+        with torch.cuda.device(dev):
+            dev_index = torch.cuda.current_device()
+            eng = self._engine_for(ih, iw, step_slots, dev_index)
+            st = self._batch_state(dev_index, step_slots, ih, iw, eng)
+            compute, copy = torch.cuda.current_stream(dev_index), st["copy"]
+            dets = torch.empty((F * S, opt.K, 6), dtype=torch.float32, device=dev)
+            h2d_done, warp_done = [None, None], [None, None]
+            for i, (fr, offsets, nbytes) in enumerate(steps):
+                b = i % 2
+                if h2d_done[b] is not None:
+                    h2d_done[b].synchronize()                  # staging buffer b is free again
+                stage, pool, grown = self._staging(st, b, nbytes)
+                host = stage.numpy()
+                desc = np.empty(len(fr) * S, WARP_DESC)
+                for k, f in enumerate(fr):
+                    self._pack_frame(images[f], layouts[f], self.scales, host, offsets[k], desc[k * S:(k + 1) * S], k * spf)
+                if grown:
+                    # a new pool may reuse memory the compute stream freed with work still queued (e.g. the flip merge's maps)
+                    copy.wait_stream(compute)
+                elif warp_done[b] is not None:
+                    copy.wait_event(warp_done[b])              # the warp of step i - 2 has read device pool b
+                with torch.cuda.stream(copy):
+                    pool[:nbytes].copy_(stage[:nbytes], non_blocking=True)
+                    h2d_done[b] = torch.cuda.Event()
+                    h2d_done[b].record(copy)
+                compute.wait_event(h2d_done[b])
+                B = len(fr) * spf
+                self._warp(pool, desc, st["dst"])
+                warp_done[b] = torch.cuda.Event()
+                warp_done[b].record(compute)
+                clock.lap("pre")
+                _, d = self._forward(st["dst"][:B], out=st["out"], maps=False)
+                clock.lap("net")
+                dets[fr.start * S:fr.stop * S].copy_(d)
+                clock.lap("dec")
+            results = self._merge_on_device(dets, metas, clock)
+        out = clock.result(None)
+        return [dict(out, results=r, **{k: out[k] / F for k in ("tot",) + _Stages.KEYS}) for r in results]
+
+    def _batch_frames(self, frames):
+        """run_batch's inputs checked and loaded: uint8 HWC 3-channel arrays as they are, paths through cv2.imread."""
+        if not self.opt.fix_res:
+            raise ValueError("run_batch needs fix_res: without it every input size compiles its own engine; use run() for keep_res")
+        for f in frames:
+            if isinstance(f, np.ndarray):
+                if f.dtype != np.uint8 or f.ndim != 3 or f.shape[2] != 3:
+                    raise ValueError("run_batch takes uint8 HWC 3-channel frames, got %s %s" % (f.dtype, f.shape))
+            elif not isinstance(f, str):
+                raise ValueError("run_batch takes uint8 arrays or image paths, not %s (prefetched dicts go through run())"
+                                 % type(f).__name__)
+        images = []
+        for f in frames:
+            if isinstance(f, str):
+                import cv2
+                image = cv2.imread(f)
+                if image is None:
+                    raise ValueError("run_batch: cannot read image %r" % f)
+                f = image
+            images.append(f)
+        return images
+
+    def _batch_state(self, dev, step_slots, ih, iw, eng):
+        """run_batch's device buffers, kept between calls so the engine replays the same graphs: the warp's destination batch,
+        the engine's outputs, the copy stream and the two staging buffers (pinned host + device pool)."""
+        key = (dev, step_slots, ih, iw)
+        st = getattr(self, "_batch", None)
+        if st is None or st["key"] != key:
+            Ho, Wo, cat = eng.plan.out_H, eng.plan.out_W, eng.plan.cat
+            f32 = lambda *shape: torch.empty(shape, dtype=torch.float32, device=dev)
+            staging = st["staging"] if st is not None and st["key"][0] == dev else [(None, None), (None, None)]
+            st = {"key": key, "dst": torch.empty((step_slots, ih, iw, 3), dtype=torch.uint8, device=dev),
+                  "out": {"hm": f32(step_slots, cat, Ho, Wo), "wh": f32(step_slots, 2, Ho, Wo), "reg": f32(step_slots, 2, Ho, Wo),
+                          "dets": f32(step_slots, self.opt.K, 6),
+                          "inds": torch.empty((step_slots, self.opt.K), dtype=torch.int32, device=dev)},
+                  "copy": torch.cuda.Stream(dev), "staging": staging}
+            self._batch = st
+        return st
+
+    def _staging(self, st, b, nbytes):
+        """Staging buffer b (pinned host, device pool) of at least nbytes, grown by half again when too small.  Returns
+        (stage, pool, grown)."""
+        stage, pool = st["staging"][b]
+        grown = stage is None or stage.numel() < nbytes
+        if grown:
+            size = max(nbytes, (stage.numel() * 3 // 2) if stage is not None else 0)
+            stage = torch.empty(size, dtype=torch.uint8, pin_memory=True)
+            pool = torch.empty(size, dtype=torch.uint8, device=st["dst"].device)
+            st["staging"][b] = (stage, pool)
+        return stage, pool, grown
 
 
 MERGE_MAX_ROWS = 1024          # CDN_SOFT_NMS_MAX_LEN: test scales x K rows per image that cdn_ctdet_merge takes
@@ -507,3 +667,24 @@ def plan_scale_batches(sizes):
     for i, hw in enumerate(sizes):
         groups.setdefault(tuple(int(v) for v in hw), []).append(i)
     return list(groups.items())
+
+
+
+def plan_frame_steps(source_bytes, slots_per_frame, max_batch, align=16):
+    """run_batch's engine steps.  source_bytes[i]: the byte sizes of frame i's source images (one per test scale), which take
+    slots_per_frame engine slots.  A step holds max(max_batch, slots_per_frame) slots and only whole frames, in frame order;
+    inside a step every source image starts at a multiple of `align` bytes of the step's pool.  Returns
+    [(frames, offsets, pool_bytes)]: frames a range of frame indices, offsets[k][j] the pool offset of source j of the step's
+    k-th frame."""
+    per_step = max(int(max_batch), slots_per_frame) // slots_per_frame
+    steps = []
+    for f0 in range(0, len(source_bytes), per_step):
+        frames = range(f0, min(f0 + per_step, len(source_bytes)))
+        offsets, end = [], 0
+        for i in frames:
+            offsets.append([])
+            for nb in source_bytes[i]:
+                offsets[-1].append(end)
+                end += -(-int(nb) // align) * align
+        steps.append((frames, offsets, end))
+    return steps

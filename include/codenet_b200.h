@@ -130,6 +130,25 @@ int cdn_deform_layer_destroy(cdn_deform_layer* layer);
  * detections ordered by class, original (score) order inside a class; d_counts [B][num_classes]. */
 int cdn_warp_affine_u8(const uint8_t* d_src, int H, int W, const double* M6, uint8_t* d_dst, int dst_h, int dst_w, int flip_copy,
                        cdn_stream_t stream);
+
+/* cdn_warp_affine_u8_batch: the same warpAffine for a ragged batch in one launch.  d_pool is a device byte pool holding source
+ * frames of any sizes back to back (uint8 HWC [src_h][src_w][3] at src_offset, any byte offset); h_desc[n] is a HOST array with
+ * one descriptor per output image: slot dst_slot of d_dst [dst_slots][dst_h][dst_w][3] receives
+ * cv2.warpAffine(frame, M, (dst_w, dst_h), flags=cv2.INTER_LINEAR) bit for bit, and slot mirror_slot (-1 = none) its mirror
+ * image (--flip_test).  Every argument is checked on the host before anything is launched (null pointers, n < 0, non-positive
+ * sizes, a negative offset, slots outside [0, dst_slots)).  The matrices are inverted on the host and the descriptors travel as
+ * kernel parameters (up to CDN_WARP_DESC_PER_LAUNCH per launch, more descriptors take several launches): no workspace, no
+ * allocation, no synchronisation, so the call can be captured into a CUDA graph.  Slots no descriptor names are left as they
+ * are.  cdn_warp_affine_u8 is the one-descriptor call {0, H, W, M6, 0, flip_copy ? 1 : -1} with dst_slots = 1 + flip_copy. */
+typedef struct cdn_warp_desc {
+  long long src_offset;              /* byte offset of the source frame in d_pool */
+  int src_h, src_w;
+  double M[6];                       /* the 2x3 source -> destination matrix cv2.warpAffine receives, row major */
+  int dst_slot, mirror_slot;
+} cdn_warp_desc;
+#define CDN_WARP_DESC_PER_LAUNCH 454
+int cdn_warp_affine_u8_batch(const uint8_t* d_pool, const cdn_warp_desc* h_desc, int n, uint8_t* d_dst, int dst_slots, int dst_h,
+                             int dst_w, cdn_stream_t stream);
 int cdn_ctdet_group_by_class(const float* d_dets, int batch, int K, int num_classes, float* d_out, int32_t* d_counts,
                              cdn_stream_t stream);
 
