@@ -119,6 +119,9 @@ EXPORTS = {
     "cdn_engine_run_host_u8": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int, C.c_void_p, C.c_void_p]),
     "cdn_warp_affine_u8": (C.c_int, [C.c_void_p, C.c_int, C.c_int, C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_void_p]),
     "cdn_warp_affine_u8_batch": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int, C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_void_p]),
+    "cdn_jpeg_parse": (C.c_int, [C.c_void_p, C.c_int64, C.c_void_p]),
+    "cdn_jpeg_decode_batch": (C.c_int, [C.c_void_p, C.c_int64, C.c_void_p, C.c_void_p, C.c_int, C.c_void_p, C.c_int64, C.c_void_p,
+                                        C.c_int64, C.c_void_p, C.c_void_p]),
     "cdn_ctdet_group_by_class": (C.c_int, [C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p]),
     "cdn_soft_nms": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_float, C.c_float, C.c_float, C.c_int, C.c_void_p,
                                C.c_void_p]),

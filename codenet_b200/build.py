@@ -6,7 +6,7 @@ import sys
 HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 LIB = os.path.join(HERE, "libcodenet_b200.so")
-SOURCES = ["engine.cu", "pw_gemm.cu", "heads_fused.cu", "unit_fused.cu", "unit_s2_fused.cu", "unit_fused_ws.cu", "dw.cu", "dw_tma.cu", "deform_tile.cu", "stem.cu", "prepost.cu", "decode.cu", "deform_f32.cu", "f32_net.cu", "pw_tf32.cu", "merge.cu"]
+SOURCES = ["engine.cu", "pw_gemm.cu", "heads_fused.cu", "unit_fused.cu", "unit_s2_fused.cu", "unit_fused_ws.cu", "dw.cu", "dw_tma.cu", "deform_tile.cu", "stem.cu", "prepost.cu", "decode.cu", "deform_f32.cu", "f32_net.cu", "pw_tf32.cu", "merge.cu", "jpeg.cu"]
 NVCC = os.environ.get("NVCC", "/usr/local/cuda/bin/nvcc")
 FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo", "-O3", "-std=c++17", "--expt-relaxed-constexpr",
          "-Xcompiler", "-fPIC", "-Xcompiler", "-O2", "-Xptxas", "-v", "-Xcudafe", "--diag_suppress=177"]

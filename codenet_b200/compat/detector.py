@@ -430,11 +430,12 @@ class CtdetDetector:
             self._warp(torch.from_numpy(pool).to(dev), desc, dst)
         return dst, [m for _, _, _, m in layout]
 
-    def _merge_on_device(self, dets, metas, clock):
+    def _merge_on_device(self, dets, metas, clock, tail=None):
         """post_process of every scale + merge_outputs for the detections [F*S, K, 6] of F images' S test scales (image-major,
         scale-minor; metas likewise): one post-affine with the per-slot transforms, one grouping, one cdn_ctdet_merge over the F
         images and one copy back.  Returns the F results.  When S x K exceeds the device merge's segment limit the per-scale
-        post_process and the host merge_outputs take over, image by image."""
+        post_process and the host merge_outputs take over, image by image.  `tail` (a device int32 tensor) comes back in the
+        same copy: then (results, tail as numpy) is returned."""
         import ctypes as C
         from .. import _lib
         S, K, nc = len(self.scales), dets.shape[1], self.num_classes
@@ -446,14 +447,15 @@ class CtdetDetector:
                 clock.lap("post")
                 results.append(self.merge_outputs(per_scale))
                 clock.lap("merge")
-            return results
+            return results if tail is None else (results, tail.cpu().numpy())
         d = dets.detach().to(self.opt.device, torch.float32).contiguous().clone()
         t = np.ascontiguousarray(np.stack([get_affine_transform(m['c'], m['s'], 0, (m['out_width'], m['out_height']), inv=1).reshape(6)
                                            for m in metas]), dtype=np.float64)
         g = torch.empty_like(d)
         counts = torch.empty((F * S, nc), dtype=torch.int32, device=d.device)
         R = S * K * 5                                                               # merged rows of one image
-        buf = torch.empty(F * (R + nc), dtype=torch.float32, device=d.device)      # rows, then the class counts (int32)
+        extra = 0 if tail is None else tail.numel()
+        buf = torch.empty(F * (R + nc) + extra, dtype=torch.float32, device=d.device)   # rows, the class counts (int32), tail
         divisors = np.ascontiguousarray(self.scales, dtype=np.float32)
         with torch.cuda.device(d.device):
             st = C.c_void_p(torch.cuda.current_stream(d.device).cuda_stream)
@@ -465,15 +467,17 @@ class CtdetDetector:
             _lib.check(L.cdn_ctdet_merge(C.c_void_p(g.data_ptr()), C.c_void_p(counts.data_ptr()), F, S, K, nc,
                                          C.c_void_p(divisors.ctypes.data), int(bool(self.opt.nms)), self.max_per_image,
                                          C.c_void_p(buf.data_ptr()), C.c_void_p(buf[F * R:].data_ptr()), st))
+            if extra:
+                buf[F * (R + nc):].view(torch.int32).copy_(tail)
         host = buf.cpu().numpy()
-        cnts = host[F * R:].view(np.int32).reshape(F, nc)
+        cnts = host[F * R:F * (R + nc)].view(np.int32).reshape(F, nc)
         results = []
         for f in range(F):
             rows, cnt = host[f * R:(f + 1) * R].reshape(-1, 5), cnts[f]
             ends = np.cumsum(cnt)
             results.append({j + 1: rows[ends[j] - cnt[j]:ends[j]] for j in range(nc)})
         clock.lap("merge")
-        return results
+        return results if tail is None else (results, host[F * (R + nc):].view(np.int32).copy())
 
     def _run_float(self, image, prepared, clock):
         """run() of the unquantised model: one network call per scale as before (its uint8 normalisation runs in torch fp32,
@@ -536,34 +540,46 @@ class CtdetDetector:
         return clock.result(self._merge_on_device(torch.cat(dets, 0), metas, clock)[0])
 
     def run_batch(self, frames):
-        """run() for many raw frames: frames is a list of uint8 HWC 3-channel arrays and/or image paths (cv2.imread).  Returns
-        one dict per frame in run()'s format; element i's results are run(frames[i])'s, and the stage timers are the call's
-        totals divided evenly across its frames (summed over frames they give the wall time).
+        """run() for many frames: frames is a list of uint8 HWC 3-channel arrays, image paths and/or encoded images (bytes,
+        bytearray, memoryview, 1-D uint8 arrays).  Returns one dict per frame in run()'s format; element i's results are
+        run(frames[i])'s (run() reads a path with cv2.imread), and the stage timers are the call's totals divided evenly across
+        its frames (summed over frames they give the wall time).  Paths are read as bytes: the file read is the "load" timer.
 
         Engine steps of max(opt.max_batch, slots of one frame) slots hold whole frames, frame-major, every frame's slots
         scale-major with each --flip_test mirror right after its image (plan_frame_steps).  Per step the raw frames and their
         host cv2.resize copies (scales other than 1) are packed into a pinned staging buffer, sent with one copy on a copy
-        stream, and one cdn_warp_affine_u8_batch launch writes every slot; then the engine, the flip merge and decode.  Two
-        staging buffers, kept on the detector, let the packing and copy of step n + 1 overlap the compute of step n.  After the
-        last step one post-affine, grouping, cdn_ctdet_merge over all frames and one copy back (_merge_on_device).
+        stream, and one cdn_warp_affine_u8_batch launch writes every slot; then the engine, the flip merge and decode.  When
+        the one test scale is 1 and a step holds at least JPEG_DEVICE_MIN_FRAMES frames, the JPEG streams the device takes
+        (cdn_jpeg_parse) go up compressed in the same staging copy,
+        with their descriptors, and one cdn_jpeg_decode_batch call decodes them into the device pool the warp reads; other
+        encoded inputs are decoded by cv2 on the host first.  Two staging buffers, kept on the detector, let the packing and
+        copy of step n + 1 overlap the compute of step n.  After the last step one post-affine, grouping, cdn_ctdet_merge over
+        all frames and one copy back (_merge_on_device), which also brings the decode status of every device-decoded frame:
+        a frame the device flagged (corrupt data) is decoded by cv2 and re-run through run().
         Needs fix_res (the engine is compiled for one input size; run() is the path for keep_res); prefetched dicts go through
         run().  The unquantised model runs run() frame by frame."""
+        from .. import jpeg
         clock = _Stages()
-        images = self._batch_frames(frames)
-        if not images:
+        items = self._batch_frames(frames)
+        if not items:
             return []
         if self.float_model:
-            return [self.run(image) for image in images]
+            return [self.run(image) for image, _, _ in items]
         clock.lap("load")
         opt, dev = self.opt, self.opt.device
         n = 2 if opt.flip_test else 1
-        S, F, ih, iw = len(self.scales), len(images), opt.input_h, opt.input_w
+        S, F, ih, iw = len(self.scales), len(items), opt.input_h, opt.input_w
         spf = n * S
-        layouts = [self._frame_layout(im.shape[0], im.shape[1], self.scales) for im in images]
+        shapes = [im.shape[:2] if im is not None else (int(d[0]["height"]), int(d[0]["width"])) for im, _, d in items]
+        layouts = [self._frame_layout(h, w, self.scales) for h, w in shapes]
         metas = [m for layout in layouts for _, _, _, m in layout]
         max_batch = getattr(opt, "max_batch", 1)
-        steps = plan_frame_steps([[sh * sw * 3 for sh, sw, _, _ in layout] for layout in layouts], spf, max_batch)
+        # a JPEG stream is staged after the raw sources of its step (device decoding implies one test scale)
+        steps = plan_frame_steps([[0] if items[f][0] is None else [sh * sw * 3 for sh, sw, _, _ in layouts[f]] for f in range(F)],
+                                 spf, max_batch)
         step_slots = max(int(max_batch), spf)
+        on_dev = [f for f in range(F) if items[f][0] is None]
+        rank = {f: k for k, f in enumerate(on_dev)}
         from .._lib import WARP_DESC
         with torch.cuda.device(dev):
             dev_index = torch.cuda.current_device()
@@ -571,28 +587,53 @@ class CtdetDetector:
             st = self._batch_state(dev_index, step_slots, ih, iw, eng)
             compute, copy = torch.cuda.current_stream(dev_index), st["copy"]
             dets = torch.empty((F * S, opt.K, 6), dtype=torch.float32, device=dev)
+            status = torch.empty(len(on_dev), dtype=torch.int32, device=dev)
             h2d_done, warp_done = [None, None], [None, None]
             for i, (fr, offsets, nbytes) in enumerate(steps):
                 b = i % 2
                 if h2d_done[b] is not None:
                     h2d_done[b].synchronize()                  # staging buffer b is free again
-                stage, pool, grown = self._staging(st, b, nbytes)
+                jf = [f for f in fr if items[f][0] is None]
+                staged = pool_bytes = nbytes
+                if jf:
+                    # staged: raw sources, the descriptor table, the streams; the device pool goes on with the decoded frames
+                    table = -(-nbytes // jpeg.WS_ALIGN) * jpeg.WS_ALIGN
+                    desc = np.concatenate([items[f][2] for f in jf])
+                    soffs, staged, out_end, ws_bytes = jpeg.layout(desc, table + desc.nbytes, [items[f][1].size for f in jf], 0)
+                    out_base = -(-staged // jpeg.WS_ALIGN) * jpeg.WS_ALIGN
+                    desc["out_offset"] += out_base
+                    pool_bytes = out_base + out_end
+                stage, pool, grown = self._staging(st, b, staged, pool_bytes)
                 host = stage.numpy()
-                desc = np.empty(len(fr) * S, WARP_DESC)
+                wdesc = np.empty(len(fr) * S, WARP_DESC)
                 for k, f in enumerate(fr):
-                    self._pack_frame(images[f], layouts[f], self.scales, host, offsets[k], desc[k * S:(k + 1) * S], k * spf)
+                    image, data, _ = items[f]
+                    if image is not None:
+                        self._pack_frame(image, layouts[f], self.scales, host, offsets[k], wdesc[k * S:(k + 1) * S], k * spf)
+                    else:
+                        j = jf.index(f)
+                        host[soffs[j]:soffs[j] + data.size] = data
+                        (sh, sw, M, _), = layouts[f]
+                        wdesc[k] = (desc[j]["out_offset"], sh, sw, np.asarray(M, np.float64).reshape(6), k * spf,
+                                    k * spf + 1 if n == 2 else -1)
+                if jf:
+                    host[table:table + desc.nbytes] = desc.view(np.uint8)
                 if grown:
                     # a new pool may reuse memory the compute stream freed with work still queued (e.g. the flip merge's maps)
                     copy.wait_stream(compute)
                 elif warp_done[b] is not None:
                     copy.wait_event(warp_done[b])              # the warp of step i - 2 has read device pool b
                 with torch.cuda.stream(copy):
-                    pool[:nbytes].copy_(stage[:nbytes], non_blocking=True)
+                    pool[:staged].copy_(stage[:staged], non_blocking=True)
                     h2d_done[b] = torch.cuda.Event()
                     h2d_done[b].record(copy)
                 compute.wait_event(h2d_done[b])
                 B = len(fr) * spf
-                self._warp(pool, desc, st["dst"])
+                if jf:
+                    ws = self._jpeg_workspace(st, ws_bytes)
+                    jpeg.decode_batch(pool.data_ptr(), pool.numel(), desc, pool.data_ptr() + table, ws.data_ptr(), ws.numel(),
+                                      pool.data_ptr(), pool.numel(), status[rank[jf[0]]:].data_ptr(), compute.cuda_stream)
+                self._warp(pool, wdesc, st["dst"])
                 warp_done[b] = torch.cuda.Event()
                 warp_done[b].record(compute)
                 clock.lap("pre")
@@ -600,31 +641,64 @@ class CtdetDetector:
                 clock.lap("net")
                 dets[fr.start * S:fr.stop * S].copy_(d)
                 clock.lap("dec")
-            results = self._merge_on_device(dets, metas, clock)
+            results, bad = self._merge_on_device(dets, metas, clock, tail=status)
+        for k in np.flatnonzero(bad):
+            # corrupt data the device flagged: what cv2.imread + run() give for the frame
+            f = on_dev[k]
+            redo = self.run(jpeg.imdecode_host(items[f][1]))
+            results[f] = redo["results"]
+            for key in _Stages.KEYS:
+                clock.t[key] += redo[key]
+            clock.mark = time.time()
         out = clock.result(None)
         return [dict(out, results=r, **{k: out[k] / F for k in ("tot",) + _Stages.KEYS}) for r in results]
 
     def _batch_frames(self, frames):
-        """run_batch's inputs checked and loaded: uint8 HWC 3-channel arrays as they are, paths through cv2.imread."""
+        """run_batch's inputs checked and loaded -> [(image, encoded bytes, JPEG descriptor)]: uint8 HWC 3-channel arrays as
+        they are (image, None, None); paths (read as bytes) and encoded images as (None, bytes, descriptor) when the device
+        decodes them (the quantised model, test_scales == [1], at least JPEG_DEVICE_MIN_FRAMES frames per engine step,
+        cdn_jpeg_parse accepts the stream), else decoded by cv2.imdecode, which is what cv2.imread does after reading the file
+        (image, None, None)."""
+        from .. import jpeg
         if not self.opt.fix_res:
             raise ValueError("run_batch needs fix_res: without it every input size compiles its own engine; use run() for keep_res")
         for f in frames:
             if isinstance(f, np.ndarray):
-                if f.dtype != np.uint8 or f.ndim != 3 or f.shape[2] != 3:
-                    raise ValueError("run_batch takes uint8 HWC 3-channel frames, got %s %s" % (f.dtype, f.shape))
-            elif not isinstance(f, str):
-                raise ValueError("run_batch takes uint8 arrays or image paths, not %s (prefetched dicts go through run())"
-                                 % type(f).__name__)
-        images = []
+                if f.dtype != np.uint8 or not (f.ndim == 1 or (f.ndim == 3 and f.shape[2] == 3)):
+                    raise ValueError("run_batch takes uint8 HWC 3-channel frames or 1-D uint8 encoded images, got %s %s"
+                                     % (f.dtype, f.shape))
+            elif not isinstance(f, (str, bytes, bytearray, memoryview)):
+                raise ValueError("run_batch takes uint8 arrays, image paths or encoded images, not %s (prefetched dicts go "
+                                 "through run())" % type(f).__name__)
+        # one restart interval decodes serially in one thread, so a device decode call costs about one frame's entropy decode
+        # (13-41 ms for 500x375 q75-q95 on a B200) whatever the number of frames: it pays from JPEG_DEVICE_MIN_FRAMES per step
+        spf = len(self.opt.test_scales) * (2 if self.opt.flip_test else 1)
+        per_step = max(int(getattr(self.opt, "max_batch", 1)), spf) // spf
+        device_jpeg = (self.opt.resume_quantize and list(self.opt.test_scales) == [1] and
+                       min(per_step, len(frames)) >= JPEG_DEVICE_MIN_FRAMES)
+        items = []
         for f in frames:
+            if isinstance(f, np.ndarray) and f.ndim == 3:
+                items.append((f, None, None))
+                continue
             if isinstance(f, str):
-                import cv2
-                image = cv2.imread(f)
-                if image is None:
-                    raise ValueError("run_batch: cannot read image %r" % f)
-                f = image
-            images.append(f)
-        return images
+                try:
+                    with open(f, "rb") as fh:
+                        data = np.frombuffer(fh.read(), np.uint8)
+                except OSError:
+                    raise ValueError("run_batch: cannot read image %r" % f) from None
+            else:
+                data = jpeg.as_bytes(f)
+            if device_jpeg:
+                rc, desc = jpeg.parse(data)
+                if rc == 0:
+                    items.append((None, data, desc))
+                    continue
+            try:
+                items.append((jpeg.imdecode_host(data), None, None))
+            except ValueError:
+                raise ValueError("run_batch: cannot read image %s" % (repr(f) if isinstance(f, str) else "(%d bytes)" % data.size)) from None
+        return items
 
     def _batch_state(self, dev, step_slots, ih, iw, eng):
         """run_batch's device buffers, kept between calls so the engine replays the same graphs: the warp's destination batch,
@@ -643,20 +717,36 @@ class CtdetDetector:
             self._batch = st
         return st
 
-    def _staging(self, st, b, nbytes):
-        """Staging buffer b (pinned host, device pool) of at least nbytes, grown by half again when too small.  Returns
-        (stage, pool, grown)."""
+    def _staging(self, st, b, nbytes, pool_bytes=None):
+        """Staging buffer b: pinned host memory of at least nbytes and a device pool of at least pool_bytes (default nbytes; the
+        pool also holds what the device writes after the copied bytes, the decoded JPEG frames), each grown by half again when
+        too small.  Returns (stage, pool, grown), grown when the device pool is new."""
+        pool_bytes = nbytes if pool_bytes is None else pool_bytes
         stage, pool = st["staging"][b]
-        grown = stage is None or stage.numel() < nbytes
+        if stage is None or stage.numel() < nbytes:
+            stage = torch.empty(max(nbytes, (stage.numel() * 3 // 2) if stage is not None else 0), dtype=torch.uint8, pin_memory=True)
+        grown = pool is None or pool.numel() < pool_bytes
         if grown:
-            size = max(nbytes, (stage.numel() * 3 // 2) if stage is not None else 0)
-            stage = torch.empty(size, dtype=torch.uint8, pin_memory=True)
+            size = max(pool_bytes, (pool.numel() * 3 // 2) if pool is not None else 0)
             pool = torch.empty(size, dtype=torch.uint8, device=st["dst"].device)
-            st["staging"][b] = (stage, pool)
+        st["staging"][b] = (stage, pool)
         return stage, pool, grown
+
+    def _jpeg_workspace(self, st, nbytes):
+        """cdn_jpeg_decode_batch's workspace (coefficients, component planes), kept with the staging buffers and grown by half
+        again when too small.  Only the compute stream uses it."""
+        ws = st.get("jpeg_ws")
+        if ws is None or ws.numel() < nbytes:
+            ws = torch.empty(max(nbytes, (ws.numel() * 3 // 2) if ws is not None else 0), dtype=torch.uint8, device=st["dst"].device)
+            st["jpeg_ws"] = ws
+        return ws
 
 
 MERGE_MAX_ROWS = 1024          # CDN_SOFT_NMS_MAX_LEN: test scales x K rows per image that cdn_ctdet_merge takes
+# frames per run_batch step from which JPEGs are decoded on the device rather than by cv2 on the host: on one B200 (1000 W) with
+# 500x375 4:2:0 files the device decode lost at 16 frames per step and at 32 frames at q95, and won from 64 frames per step
+# (profiles/r04_jpeg_decode.json, run_batch rows "paths_device_decode" against "host_imread_then_arrays")
+JPEG_DEVICE_MIN_FRAMES = 48
 
 
 def plan_scale_batches(sizes):

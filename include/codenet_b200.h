@@ -152,6 +152,76 @@ int cdn_warp_affine_u8_batch(const uint8_t* d_pool, const cdn_warp_desc* h_desc,
 int cdn_ctdet_group_by_class(const float* d_dets, int batch, int K, int num_classes, float* d_out, int32_t* d_counts,
                              cdn_stream_t stream);
 
+/* ---- baseline JPEG decoding on the device (csrc/jpeg.cu, DESIGN.md section 9) -------------------------------------------
+ * cdn_jpeg_parse (HOST only, needs no device) reads the marker segments of one encoded image of nbytes bytes and fills *out.
+ * Returns 0 when the device decodes the stream, a positive CDN_JPEG_HOST_* reason when only a host decoder does (the caller
+ * decodes it with cv2.imdecode), or a negative CDN_JPEG_ERR_* when it is not a parseable JPEG.  Every read is bounded by
+ * nbytes and every table is checked: malformed input returns a status.  The device takes SOF0/SOF1 8-bit, gray or YCbCr (the
+ * libjpeg colour-space rule) with luma sampling 1x1, 2x1 or 2x2 and chroma 1x1, one interleaved scan holding every component,
+ * 8- or 16-bit quantisation tables, any restart interval, and no Exif orientation other than 1.
+ *
+ * cdn_jpeg_decode_batch decodes n parsed frames in one call on `stream`: what cv2.imdecode(buf, cv2.IMREAD_COLOR) returns,
+ * element for element, as uint8 BGR HWC [height][width][3] at out_offset of d_out (the source format of
+ * cdn_warp_affine_u8_batch).  h_frames is the HOST array the caller filled (cdn_jpeg_parse, then data_offset, out_offset,
+ * ws_offset) and d_frames a device copy of the same n descriptors, complete before the work on `stream` runs.  Stream i lies at
+ * d_pool[data_offset, data_offset + nbytes); its workspace (restart offsets, int16 coefficient blocks, component planes) at
+ * d_ws[ws_offset, ws_offset + ws_bytes), 256-byte aligned.  Every descriptor is checked on the host against pool_bytes,
+ * ws_bytes and out_bytes first; then four kernels run (restart-marker index, entropy decode, dequantise + islow IDCT,
+ * upsample + colour).  No allocation and no synchronisation: the call can be captured.  d_status[i] receives 0 when frame i
+ * decoded, else CDN_JPEG_BAD_* bits: its output bytes are then undefined and the frame must be decoded on the host. */
+#define CDN_JPEG_HOST_PROCESS 1        /* progressive, lossless, hierarchical or arithmetic-coded */
+#define CDN_JPEG_HOST_PRECISION 2      /* not 8-bit samples */
+#define CDN_JPEG_HOST_COLOR 3          /* neither 1 component nor 3 in YCbCr (CMYK, YCCK, RGB) */
+#define CDN_JPEG_HOST_SAMPLING 4       /* 3 components other than 4:4:4, 4:2:2 or 4:2:0 */
+#define CDN_JPEG_HOST_SCAN 5           /* several scans, a scan without every component, DNL, undefined tables */
+#define CDN_JPEG_HOST_ORIENTATION 6    /* an Exif orientation other than 1 (cv2 rotates), or an Exif block it cannot read */
+#define CDN_JPEG_HOST_SIZE 7           /* more than 2^26 pixels, or a stream of 2 GB or more */
+#define CDN_JPEG_ERR_NOT_JPEG (-1)     /* no SOI marker */
+#define CDN_JPEG_ERR_TRUNCATED (-2)    /* the headers end before the scan */
+#define CDN_JPEG_ERR_SEGMENT (-3)      /* a marker segment with an impossible length or content */
+#define CDN_JPEG_ERR_TABLE (-4)        /* a quantisation or Huffman table libjpeg rejects */
+#define CDN_JPEG_BAD_CODE 1            /* an invalid Huffman code or a run past coefficient 63 */
+#define CDN_JPEG_BAD_END 2             /* the data of a restart interval ends (marker or end of scan) before its last MCU */
+#define CDN_JPEG_BAD_RESTART 4         /* restart markers missing, extra or out of sequence */
+#define CDN_JPEG_BAD_RANGE 8           /* coefficients or IDCT outputs outside the window where libjpeg-turbo's C and SIMD agree */
+#define CDN_JPEG_LOOKAHEAD 8
+
+typedef struct cdn_jpeg_huff {         /* jpeg_make_d_derived_tbl's decoding form of one Huffman table */
+  int32_t maxcode[18];                 /* largest code of each length 1..16, -1 if none; maxcode[17] = 0xFFFFF */
+  int32_t valoffset[18];               /* huffval index of a code of length l = code + valoffset[l] */
+  uint16_t look[1 << CDN_JPEG_LOOKAHEAD];  /* next 8 bits -> (length << 8) | symbol, 0 when the code is longer */
+  uint8_t huffval[256];
+} cdn_jpeg_huff;
+
+typedef struct cdn_jpeg_frame {
+  /* filled by cdn_jpeg_parse */
+  int32_t width, height, ncomp;        /* ncomp 1 (gray) or 3 (YCbCr) */
+  int32_t hmax, vmax;                  /* luma sampling factors (1 for gray) */
+  int32_t mcux, mcuy;                  /* MCU grid */
+  int32_t restart_interval;            /* MCUs per entropy-coded segment, 0 = none */
+  int32_t nsegments;                   /* entropy-coded segments (restart intervals) */
+  int32_t pad0;
+  int64_t nbytes;                      /* bytes of the stream */
+  int64_t scan_offset, scan_end;       /* entropy-coded bytes [scan_offset, scan_end) of the stream */
+  int32_t comp_h[3], comp_v[3];        /* blocks per MCU of each component */
+  int32_t comp_bw[3], comp_bh[3];      /* block grid of each component */
+  int32_t comp_dw[3], comp_dh[3];      /* downsampled (valid) size of each component */
+  int32_t comp_dc[3], comp_ac[3];      /* Huffman table of each component: huff[0..1] DC, huff[2..3] AC */
+  int64_t ws_bytes;                    /* workspace this frame needs */
+  int64_t coef_rel, plane_rel[3];      /* workspace layout: restart offsets at 0, coefficients, planes */
+  uint16_t qt[3][64];                  /* dequantisation table of each component, natural order */
+  cdn_jpeg_huff huff[4];
+  /* filled by the caller */
+  int64_t data_offset;                 /* stream position in d_pool */
+  int64_t out_offset;                  /* BGR frame position in d_out */
+  int64_t ws_offset;                   /* workspace position in d_ws (a multiple of 256) */
+} cdn_jpeg_frame;
+
+int cdn_jpeg_parse(const uint8_t* data, int64_t nbytes, cdn_jpeg_frame* out);
+int cdn_jpeg_decode_batch(const uint8_t* d_pool, int64_t pool_bytes, const cdn_jpeg_frame* h_frames,
+                          const cdn_jpeg_frame* d_frames, int n, uint8_t* d_ws, int64_t ws_bytes, uint8_t* d_out,
+                          int64_t out_bytes, int32_t* d_status, cdn_stream_t stream);
+
 /* ---- multi-scale merge and soft-NMS (lib/detectors/ctdet.py:59-74, lib/models/external/nms.pyx:77-170) ---------------
  * cdn_soft_nms: the reference's soft_nms on n_seg independent segments of d_boxes [rows][5] (x1, y1, x2, y2, score), segment g =
  * rows [d_seg_off[g], d_seg_off[g+1]) (device int32, non-overlapping), each modified IN PLACE exactly as compat.soft_nms
