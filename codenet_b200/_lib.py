@@ -41,6 +41,7 @@ WARP_DESC = np.dtype([("src_offset", np.int64), ("src_h", np.int32), ("src_w", n
                       ("dst_slot", np.int32), ("mirror_slot", np.int32)])
 assert WARP_DESC.itemsize == 72
 WARP_DESC_PER_LAUNCH = 454         # CDN_WARP_DESC_PER_LAUNCH
+WARP_F32_DESC_PER_LAUNCH = 448     # CDN_WARP_F32_DESC_PER_LAUNCH (cdn_warp_affine_u8_f32_batch)
 
 EXPORTS = {
     "cdn_last_error": (C.c_char_p, []),
@@ -119,6 +120,8 @@ EXPORTS = {
     "cdn_engine_run_host_u8": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int, C.c_void_p, C.c_void_p]),
     "cdn_warp_affine_u8": (C.c_int, [C.c_void_p, C.c_int, C.c_int, C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_void_p]),
     "cdn_warp_affine_u8_batch": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int, C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_void_p]),
+    "cdn_warp_affine_u8_f32_batch": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.c_void_p, C.c_int, C.c_void_p, C.c_int,
+                                               C.c_int, C.c_int, C.c_void_p]),
     "cdn_jpeg_parse": (C.c_int, [C.c_void_p, C.c_int64, C.c_void_p]),
     "cdn_jpeg_decode_batch": (C.c_int, [C.c_void_p, C.c_int64, C.c_void_p, C.c_void_p, C.c_int, C.c_void_p, C.c_int64, C.c_void_p,
                                         C.c_int64, C.c_void_p, C.c_void_p]),

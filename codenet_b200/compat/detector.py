@@ -5,7 +5,8 @@ freezes the activation ranges and runs forward + decode through the compiled int
 dict as the reference (`results` keyed by 1-based class id and the stage timers test.py prints, test.py:76-79).
 Only what differs from the reference lives here: engine construction, process / process_u8, the device-side box transform,
 run()'s multi-scale path (all test scales of an image in one engine batch, merge_outputs on the device: cdn_ctdet_merge) and
-run_batch() (many raw frames per engine step, their warpAffine in one cdn_warp_affine_u8_batch launch per step).
+run_batch() (many raw frames per engine step, their warpAffine in one cdn_warp_affine_u8_batch launch per step, or for the
+unquantised model one cdn_warp_affine_u8_f32_batch launch that also normalises).
 pre_process, merge_outputs and run keep the reference's contract (same inputs, outputs and timer keys) in this package's own
 decomposition (input_geometry / _Stages / group_by_class); INTEGRATION.md section 2 shows the patch for users who keep the reference's BaseDetector.
 """
@@ -198,10 +199,41 @@ class CtdetDetector:
         import cv2
         (sh, sw), (ih, iw), c, s = self.input_geometry(image.shape[0], image.shape[1], scale)
         warped = cv2.warpAffine(cv2.resize(image, (sw, sh)), get_affine_transform(c, s, 0, [iw, ih]), (iw, ih), flags=cv2.INTER_LINEAR)
-        chw = ((warped / 255. - self.mean) / self.std).astype(np.float32).transpose(2, 0, 1)[None]
+        chw = self._normalize_host(warped).transpose(2, 0, 1)[None]
         if self.opt.flip_test:
             chw = np.concatenate([chw, chw[..., ::-1]], 0)
         return torch.from_numpy(np.ascontiguousarray(chw)), self._meta(c, s, ih, iw)
+
+    def _normalize_host(self, warped):
+        """pre_process's normalisation (base_detector.py:66-68) of uint8 HWC pixels: numpy float64, rounded once to fp32."""
+        return ((warped / 255. - self.mean) / self.std).astype(np.float32)
+
+    def _normalize_device(self, images):
+        """_process_float's normalisation of uint8 [..., 3] CUDA pixels (pre_process_device's layout): torch fp32 on the device."""
+        mean = torch.as_tensor(self.mean.reshape(3), device=images.device)
+        std = torch.as_tensor(self.std.reshape(3), device=images.device)
+        return (images.float() / 255.0 - mean) / std
+
+    def _device_table(self, scale):
+        """Which normalisation run() gives test scale `scale` of a uint8 HWC frame in the unquantised model: True for
+        _normalize_device (pre_process_device: scale 1 with opt.device_pre_process), False for pre_process's _normalize_host."""
+        return scale == 1 and bool(getattr(self.opt, "device_pre_process", True))
+
+    def _table_index(self, scales, frames):
+        """cdn_warp_affine_u8_f32_batch's table index of every descriptor of `frames` frames (frame-major, scale-minor): 0 for
+        the device normalisation, 1 for the host one (_device_table, _norm_tables)."""
+        return np.tile(np.array([0 if self._device_table(s) else 1 for s in scales], np.int32), frames)
+
+    def _host_table(self):
+        """_normalize_host of the 256 byte values in every channel: numpy fp32 [3, 256]."""
+        return np.ascontiguousarray(self._normalize_host(np.repeat(_BYTES[:, None], 3, 1)[None])[0].T)
+
+    def _norm_tables(self, dev):
+        """The tables of cdn_warp_affine_u8_f32_batch, fp32 [2, 3, 256] on `dev`: [0] = _normalize_device and [1] =
+        _normalize_host of the 256 byte values in every channel, each computed by the helper itself.  Both normalisations are
+        elementwise functions of a byte and its channel, so a lookup in these tables gives exactly what they give."""
+        on_dev = self._normalize_device(torch.from_numpy(np.repeat(_BYTES[:, None], 3, 1)).to(dev)).t()
+        return torch.stack([on_dev, torch.from_numpy(self._host_table()).to(dev)]).contiguous()
 
     def pre_process_device(self, image, scale=1, meta=None):
         """pre_process for a raw uint8 HWC image at test scale 1 ON THE DEVICE: the frame is uploaded as it is and
@@ -250,14 +282,19 @@ class CtdetDetector:
 
     def _process_float(self, images, return_time):
         """process() for the unquantised model: EngineF32 forward (logits), hm.sigmoid_() as ctdet.py:32, decode on the device."""
+        if images.dtype == torch.uint8:                              # pre_process_device's layout: normalise as base_detector.py:66-68
+            images = self._normalize_device(images).permute(0, 3, 1, 2)
+        x = images.contiguous().float()
+        output, dets = self._forward_float(x)
+        torch.cuda.synchronize(x.device)
+        forward_time = time.time()
+        return (output, dets, forward_time) if return_time else (output, dets)
+
+    def _forward_float(self, x):
+        """_process_float without the synchronisation: enqueues EngineF32 (detect, or forward + the flip average + decode with
+        --flip_test) on the current stream and returns (output, dets).  x: contiguous CUDA fp32 [B,3,H,W]."""
         from ..arch import NetConfig
         from ..engine_f32 import EngineF32
-        if images.dtype == torch.uint8:                              # pre_process_device's layout: normalise as base_detector.py:66-68
-            mean = torch.as_tensor(self.mean.reshape(3), device=images.device)
-            std = torch.as_tensor(self.std.reshape(3), device=images.device)
-            images = ((images.float() / 255.0 - mean) / std).permute(0, 3, 1, 2)
-        x = images.contiguous().float()
-        B = x.shape[0]
         dev = x.device.index if x.device.index is not None else torch.cuda.current_device()
         eng = self._f32_engines.get(dev)
         if eng is None:
@@ -278,9 +315,7 @@ class CtdetDetector:
         output = {"hm": hm, "wh": wh}
         if reg is not None:
             output["reg"] = reg
-        torch.cuda.synchronize(x.device)
-        forward_time = time.time()
-        return (output, dets, forward_time) if return_time else (output, dets)
+        return output, dets
 
     def process(self, images, return_time=False):
         """images: CUDA fp32 [B,3,H,W] (the reference's tensor) or uint8 [B,H,W,3] (pre_process_device).
@@ -413,6 +448,17 @@ class CtdetDetector:
         _lib.check(_lib.load().cdn_warp_affine_u8_batch(C.c_void_p(pool.data_ptr()), C.c_void_p(desc.ctypes.data), len(desc),
                                                          C.c_void_p(dst.data_ptr()), dst.shape[0], dst.shape[1], dst.shape[2], st))
 
+    def _warp_f32(self, pool, desc, table, tables, dst):
+        """cdn_warp_affine_u8_f32_batch on the current stream: the descriptors `desc` from the device byte pool into the fp32 CUDA
+        batch dst [slots, 3, H, W], descriptor i normalised with tables[table[i]] (_norm_tables)."""
+        import ctypes as C
+        from .. import _lib
+        st = C.c_void_p(torch.cuda.current_stream(dst.device).cuda_stream)
+        table = np.ascontiguousarray(table, dtype=np.int32)
+        _lib.check(_lib.load().cdn_warp_affine_u8_f32_batch(
+            C.c_void_p(pool.data_ptr()), C.c_void_p(desc.ctypes.data), C.c_void_p(table.ctypes.data), len(desc),
+            C.c_void_p(tables.data_ptr()), tables.shape[0], C.c_void_p(dst.data_ptr()), dst.shape[0], dst.shape[2], dst.shape[3], st))
+
     def _slots_u8(self, image, scales, ih, iw):
         """The network images of `scales` of one uint8 HWC frame as one uint8 CUDA batch [slots, ih, iw, 3] (scale-major, the
         mirror after its image): the frame and its host cv2.resize copies (scales other than 1) go to the device in one byte pool
@@ -487,7 +533,7 @@ class CtdetDetector:
             if prepared is not None:
                 images = prepared['images'][scale][0]
                 meta = {k: (v.numpy()[0] if torch.is_tensor(v) else v) for k, v in prepared['meta'][scale].items()}
-            elif scale == 1 and image.dtype == np.uint8 and image.ndim == 3 and getattr(self.opt, "device_pre_process", True):
+            elif image.dtype == np.uint8 and image.ndim == 3 and self._device_table(scale):
                 images, meta = self.pre_process_device(image, scale)
             else:
                 images, meta = self.pre_process(image, scale)
@@ -548,7 +594,10 @@ class CtdetDetector:
         Engine steps of max(opt.max_batch, slots of one frame) slots hold whole frames, frame-major, every frame's slots
         scale-major with each --flip_test mirror right after its image (plan_frame_steps).  Per step the raw frames and their
         host cv2.resize copies (scales other than 1) are packed into a pinned staging buffer, sent with one copy on a copy
-        stream, and one cdn_warp_affine_u8_batch launch writes every slot; then the engine, the flip merge and decode.  When
+        stream, and one cdn_warp_affine_u8_batch launch writes every slot; then the engine, the flip merge and decode.  The
+        unquantised model takes the same steps with one cdn_warp_affine_u8_f32_batch launch instead, which writes normalised
+        fp32 NCHW slots through the 3 x 256 table run() uses for each scale (_device_table, _norm_tables), then EngineF32
+        eagerly (_forward_float).  When
         the one test scale is 1 and a step holds at least JPEG_DEVICE_MIN_FRAMES frames, the JPEG streams the device takes
         (cdn_jpeg_parse) go up compressed in the same staging copy,
         with their descriptors, and one cdn_jpeg_decode_batch call decodes them into the device pool the warp reads; other
@@ -557,14 +606,12 @@ class CtdetDetector:
         all frames and one copy back (_merge_on_device), which also brings the decode status of every device-decoded frame:
         a frame the device flagged (corrupt data) is decoded by cv2 and re-run through run().
         Needs fix_res (the engine is compiled for one input size; run() is the path for keep_res); prefetched dicts go through
-        run().  The unquantised model runs run() frame by frame."""
+        run().  JPEGs of the unquantised model are decoded by cv2 on the host."""
         from .. import jpeg
         clock = _Stages()
         items = self._batch_frames(frames)
         if not items:
             return []
-        if self.float_model:
-            return [self.run(image) for image, _, _ in items]
         clock.lap("load")
         opt, dev = self.opt, self.opt.device
         n = 2 if opt.flip_test else 1
@@ -583,7 +630,7 @@ class CtdetDetector:
         from .._lib import WARP_DESC
         with torch.cuda.device(dev):
             dev_index = torch.cuda.current_device()
-            eng = self._engine_for(ih, iw, step_slots, dev_index)
+            eng = None if self.float_model else self._engine_for(ih, iw, step_slots, dev_index)
             st = self._batch_state(dev_index, step_slots, ih, iw, eng)
             compute, copy = torch.cuda.current_stream(dev_index), st["copy"]
             dets = torch.empty((F * S, opt.K, 6), dtype=torch.float32, device=dev)
@@ -633,11 +680,17 @@ class CtdetDetector:
                     ws = self._jpeg_workspace(st, ws_bytes)
                     jpeg.decode_batch(pool.data_ptr(), pool.numel(), desc, pool.data_ptr() + table, ws.data_ptr(), ws.numel(),
                                       pool.data_ptr(), pool.numel(), status[rank[jf[0]]:].data_ptr(), compute.cuda_stream)
-                self._warp(pool, wdesc, st["dst"])
+                if self.float_model:
+                    self._warp_f32(pool, wdesc, self._table_index(self.scales, len(fr)), st["tables"], st["dst"])
+                else:
+                    self._warp(pool, wdesc, st["dst"])
                 warp_done[b] = torch.cuda.Event()
                 warp_done[b].record(compute)
                 clock.lap("pre")
-                _, d = self._forward(st["dst"][:B], out=st["out"], maps=False)
+                if self.float_model:
+                    _, d = self._forward_float(st["dst"][:B])
+                else:
+                    _, d = self._forward(st["dst"][:B], out=st["out"], maps=False)
                 clock.lap("net")
                 dets[fr.start * S:fr.stop * S].copy_(d)
                 clock.lap("dec")
@@ -702,18 +755,22 @@ class CtdetDetector:
 
     def _batch_state(self, dev, step_slots, ih, iw, eng):
         """run_batch's device buffers, kept between calls so the engine replays the same graphs: the warp's destination batch,
-        the engine's outputs, the copy stream and the two staging buffers (pinned host + device pool)."""
+        the engine's outputs, the copy stream and the two staging buffers (pinned host + device pool).  The unquantised model
+        (eng None) has an fp32 NCHW destination and the normalisation tables instead of engine outputs."""
         key = (dev, step_slots, ih, iw)
         st = getattr(self, "_batch", None)
         if st is None or st["key"] != key:
-            Ho, Wo, cat = eng.plan.out_H, eng.plan.out_W, eng.plan.cat
             f32 = lambda *shape: torch.empty(shape, dtype=torch.float32, device=dev)
             staging = st["staging"] if st is not None and st["key"][0] == dev else [(None, None), (None, None)]
-            st = {"key": key, "dst": torch.empty((step_slots, ih, iw, 3), dtype=torch.uint8, device=dev),
-                  "out": {"hm": f32(step_slots, cat, Ho, Wo), "wh": f32(step_slots, 2, Ho, Wo), "reg": f32(step_slots, 2, Ho, Wo),
-                          "dets": f32(step_slots, self.opt.K, 6),
-                          "inds": torch.empty((step_slots, self.opt.K), dtype=torch.int32, device=dev)},
-                  "copy": torch.cuda.Stream(dev), "staging": staging}
+            st = {"key": key, "copy": torch.cuda.Stream(dev), "staging": staging}
+            if self.float_model:
+                st.update(dst=f32(step_slots, 3, ih, iw), tables=self._norm_tables(dev))
+            else:
+                Ho, Wo, cat = eng.plan.out_H, eng.plan.out_W, eng.plan.cat
+                st["dst"] = torch.empty((step_slots, ih, iw, 3), dtype=torch.uint8, device=dev)
+                st["out"] = {"hm": f32(step_slots, cat, Ho, Wo), "wh": f32(step_slots, 2, Ho, Wo), "reg": f32(step_slots, 2, Ho, Wo),
+                             "dets": f32(step_slots, self.opt.K, 6),
+                             "inds": torch.empty((step_slots, self.opt.K), dtype=torch.int32, device=dev)}
             self._batch = st
         return st
 
@@ -742,6 +799,7 @@ class CtdetDetector:
         return ws
 
 
+_BYTES = np.arange(256, dtype=np.uint8)
 MERGE_MAX_ROWS = 1024          # CDN_SOFT_NMS_MAX_LEN: test scales x K rows per image that cdn_ctdet_merge takes
 # frames per run_batch step from which JPEGs are decoded on the device rather than by cv2 on the host: on one B200 (1000 W) with
 # 500x375 4:2:0 files the device decode lost at 16 frames per step and at 32 frames at q95, and won from 64 frames per step

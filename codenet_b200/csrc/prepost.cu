@@ -6,11 +6,16 @@
 //     back to back in one byte pool, one descriptor per output image.  cdn_warp_affine_u8 is its one-descriptor case.  At
 //     test scale 1 the cv2.resize in front of it is the identity, so the raw frame goes to the device as it is and the
 //     normalisation happens in the stem kernel's 3 x 256 table.
+//   * cdn_warp_affine_u8_f32_batch -- the same warp for the unquantised model, whose network takes normalised fp32 NCHW: every
+//     warped byte goes through a 3 x 256 fp32 table (the normalisation of BaseDetector.pre_process, :66-68, is a function of
+//     the byte and its channel) and is written in planes.  Both kernels call one interpolation function, so the fp32 output is
+//     the u8 kernel's output looked up, by construction.
 //   * cdn_ctdet_group_by_class -- the per-class grouping of ctdet_post_process (lib/utils/post_process.py:86-103): detections
 //     [B][K][6] reordered by class (stable, i.e. by descending score inside a class) + per-class counts, so the host only
 //     slices views.
 #include "common.cuh"
 #include <algorithm>
+#include <cstddef>
 
 // one output image: its source frame in the pool and the INVERSE (destination -> source) matrix
 struct WarpDesc { long long off; int H, W; double m[6]; int dst, mirror; };
@@ -24,6 +29,15 @@ static_assert(WARP_MAX_DESC == CDN_WARP_DESC_PER_LAUNCH, "include/codenet_b200.h
 static_assert(sizeof(cdn_warp_desc) == 72, "cdn_warp_desc layout (codenet_b200._lib.WARP_DESC)");
 struct WarpBatchParams { const uint8_t* pool; uint8_t* dst; int dh, dw, groups, pad; WarpDesc d[WARP_MAX_DESC]; };
 static_assert(sizeof(WarpBatchParams) <= 32764, "kernel parameters exceed 32764 bytes");
+// the fp32 variant: 40 bytes of header, then per descriptor its WarpDesc and the one-byte index of its normalisation table
+constexpr int WARP_F32_MAX_DESC = (32764 - 40) / (int)(sizeof(WarpDesc) + sizeof(uint8_t));
+static_assert(WARP_F32_MAX_DESC == CDN_WARP_F32_DESC_PER_LAUNCH, "include/codenet_b200.h states the descriptors per launch");
+struct WarpF32Params {
+  const uint8_t* pool; float* dst; const float* tables; int dh, dw, groups, vec;
+  WarpDesc d[WARP_F32_MAX_DESC]; uint8_t table[WARP_F32_MAX_DESC];
+};
+static_assert(offsetof(WarpF32Params, d) == 40, "WarpF32Params header");
+static_assert(sizeof(WarpF32Params) <= 32764, "kernel parameters exceed 32764 bytes");
 
 // cv::warpAffine's inversion of the 2 x 3 matrix (imgwarp.cpp), in double on the host: the same expressions on the device
 // would be contracted into FMAs and could round differently
@@ -51,19 +65,15 @@ __device__ __forceinline__ void warp_store(uint8_t* d, const uint8_t (&v)[WARP_P
   }
 }
 
-// grid (tiles of WARP_THREADS x WARP_PX pixels over the flattened dst_h x dst_w image, descriptors of this launch)
-__global__ void __launch_bounds__(WARP_THREADS) warp_affine_u8_kernel(const __grid_constant__ WarpBatchParams p) {
-  const WarpDesc& q = p.d[blockIdx.y];
-  const int t = blockIdx.x * WARP_THREADS + threadIdx.x;
-  const int y = t / p.groups, x0 = (t - y * p.groups) * WARP_PX;
-  if (y >= p.dh) return;
-  const int n = min(WARP_PX, p.dw - x0);
-  const uint8_t* src = p.pool + q.off;
+// OpenCV's fixed-point bilinear interpolation of WARP_PX consecutive destination pixels (y, x0 .. x0 + WARP_PX - 1) of one
+// descriptor, the one both warp kernels call: v[i * 3 + c] = channel c of pixel x0 + i (a pixel past the row's end is
+// computed like the others and left unstored by the caller)
+__device__ __forceinline__ void warp_pixels(const WarpDesc& q, const uint8_t* pool, int y, int x0, uint8_t (&v)[WARP_PX * 3]) {
+  const uint8_t* src = pool + q.off;
   // dst -> src map in 1/1024 pixel, as OpenCV forms it: per-column and per-row terms are rounded SEPARATELY, then summed;
   // the row term is m1 * y + m2 in two roundings (no FMA), like OpenCV's and numpy's double arithmetic
   const int X0 = __double2int_rn(__dmul_rn(__dadd_rn(__dmul_rn(q.m[1], (double)y), q.m[2]), 1024.0)) + 16;
   const int Y0 = __double2int_rn(__dmul_rn(__dadd_rn(__dmul_rn(q.m[4], (double)y), q.m[5]), 1024.0)) + 16;
-  uint8_t v[WARP_PX * 3];
 #pragma unroll
   for (int i = 0; i < WARP_PX; ++i) {
     const int x = x0 + i;
@@ -85,6 +95,17 @@ __global__ void __launch_bounds__(WARP_THREADS) warp_affine_u8_kernel(const __gr
 #pragma unroll
     for (int c = 0; c < 3; ++c) v[i * 3 + c] = (uint8_t)min(max((acc[c] + (1 << 14)) >> 15, 0), 255);
   }
+}
+
+// grid (tiles of WARP_THREADS x WARP_PX pixels over the flattened dst_h x dst_w image, descriptors of this launch)
+__global__ void __launch_bounds__(WARP_THREADS) warp_affine_u8_kernel(const __grid_constant__ WarpBatchParams p) {
+  const WarpDesc& q = p.d[blockIdx.y];
+  const int t = blockIdx.x * WARP_THREADS + threadIdx.x;
+  const int y = t / p.groups, x0 = (t - y * p.groups) * WARP_PX;
+  if (y >= p.dh) return;
+  const int n = min(WARP_PX, p.dw - x0);
+  uint8_t v[WARP_PX * 3];
+  warp_pixels(q, p.pool, y, x0, v);
   const size_t plane = (size_t)p.dh * p.dw * 3, row = (size_t)y * p.dw * 3;
   warp_store(p.dst + (size_t)q.dst * plane + row + (size_t)x0 * 3, v, n);
   if (q.mirror >= 0) {                               // the n pixels reversed, ending at column dw - 1 - x0
@@ -105,35 +126,108 @@ __global__ void __launch_bounds__(WARP_THREADS) warp_affine_u8_kernel(const __gr
   }
 }
 
-extern "C" int cdn_warp_affine_u8_batch(const uint8_t* d_pool, const cdn_warp_desc* h_desc, int n, uint8_t* d_dst, int dst_slots,
-                                        int dst_h, int dst_w, cdn_stream_t stream) {
-  CDN_CHECK(d_pool && h_desc && d_dst, CDN_ERR_INVALID, "warp_affine_batch: null pointer");
-  CDN_CHECK(n >= 0, CDN_ERR_INVALID, "warp_affine_batch: n = %d", n);
-  CDN_CHECK(dst_slots > 0 && dst_h > 0 && dst_w > 0, CDN_ERR_INVALID, "warp_affine_batch: bad destination %d x %d x %d",
-            dst_slots, dst_h, dst_w);
-  const int groups = (dst_w + WARP_PX - 1) / WARP_PX;
+// The same pixels through a 3 x 256 table into fp32 NCHW: element (slot, c, y, x) = table[c][byte the u8 kernel writes at
+// (slot, y, x, c)].  The descriptor's table is staged in shared memory; with vec (dst_w % 4 == 0, 16-byte-aligned dst) a thread
+// stores one float4 per channel plane, and one per plane of the mirror.
+__global__ void __launch_bounds__(WARP_THREADS) warp_affine_u8_f32_kernel(const __grid_constant__ WarpF32Params p) {
+  __shared__ float s_tab[3 * 256];
+  const WarpDesc& q = p.d[blockIdx.y];
+  const float* tab = p.tables + (size_t)p.table[blockIdx.y] * (3 * 256);
+  for (int i = threadIdx.x; i < 3 * 256; i += WARP_THREADS) s_tab[i] = __ldg(tab + i);
+  __syncthreads();
+  const int t = blockIdx.x * WARP_THREADS + threadIdx.x;
+  const int y = t / p.groups, x0 = (t - y * p.groups) * WARP_PX;
+  if (y >= p.dh) return;
+  const int n = min(WARP_PX, p.dw - x0);
+  uint8_t v[WARP_PX * 3];
+  warp_pixels(q, p.pool, y, x0, v);
+  const size_t plane = (size_t)p.dh * p.dw, row = (size_t)y * p.dw;
+  float* d = p.dst + (size_t)q.dst * 3 * plane + row + x0;
+  float* m = q.mirror >= 0 ? p.dst + (size_t)q.mirror * 3 * plane + row + (p.dw - x0 - n) : nullptr;   // ends at dw - 1 - x0
+#pragma unroll
+  for (int c = 0; c < 3; ++c) {
+    float f[WARP_PX];
+#pragma unroll
+    for (int i = 0; i < WARP_PX; ++i) f[i] = s_tab[c * 256 + v[i * 3 + c]];
+    if (p.vec) {
+      *reinterpret_cast<float4*>(d + c * plane) = make_float4(f[0], f[1], f[2], f[3]);
+      if (m) *reinterpret_cast<float4*>(m + c * plane) = make_float4(f[3], f[2], f[1], f[0]);
+    } else {
+#pragma unroll
+      for (int i = 0; i < WARP_PX; ++i)
+        if (i < n) {
+          d[c * plane + i] = f[i];
+          if (m) m[c * plane + n - 1 - i] = f[i];
+        }
+    }
+  }
+}
+
+// the checks both batch entry points make before anything is launched
+static int warp_batch_check(const char* who, const cdn_warp_desc* h_desc, int n, int dst_slots, int dst_h, int dst_w) {
+  CDN_CHECK(n >= 0, CDN_ERR_INVALID, "%s: n = %d", who, n);
+  CDN_CHECK(dst_slots > 0 && dst_h > 0 && dst_w > 0, CDN_ERR_INVALID, "%s: bad destination %d x %d x %d", who, dst_slots, dst_h,
+            dst_w);
+  const long long groups = ((long long)dst_w + WARP_PX - 1) / WARP_PX;
   const long long tiles = ((long long)dst_h * groups + WARP_THREADS - 1) / WARP_THREADS;
   CDN_CHECK(tiles <= 0x7fffffffLL && (long long)dst_h * groups <= 0x7fffffffLL, CDN_ERR_INVALID,
-            "warp_affine_batch: destination %d x %d too large", dst_h, dst_w);
+            "%s: destination %d x %d too large", who, dst_h, dst_w);
   for (int i = 0; i < n; ++i) {
     const cdn_warp_desc& d = h_desc[i];
     CDN_CHECK(d.src_offset >= 0 && d.src_h > 0 && d.src_w > 0, CDN_ERR_INVALID,
-              "warp_affine_batch: descriptor %d: bad source (offset %lld, %d x %d)", i, d.src_offset, d.src_h, d.src_w);
+              "%s: descriptor %d: bad source (offset %lld, %d x %d)", who, i, d.src_offset, d.src_h, d.src_w);
     CDN_CHECK(d.dst_slot >= 0 && d.dst_slot < dst_slots && d.mirror_slot >= -1 && d.mirror_slot < dst_slots, CDN_ERR_INVALID,
-              "warp_affine_batch: descriptor %d: slot %d / mirror %d outside [0, %d)", i, d.dst_slot, d.mirror_slot, dst_slots);
+              "%s: descriptor %d: slot %d / mirror %d outside [0, %d)", who, i, d.dst_slot, d.mirror_slot, dst_slots);
   }
+  return 0;
+}
+
+static void warp_fill(const cdn_warp_desc& d, WarpDesc& q) {
+  q.off = d.src_offset; q.H = d.src_h; q.W = d.src_w; q.dst = d.dst_slot; q.mirror = d.mirror_slot;
+  warp_invert(d.M, q.m);
+}
+
+extern "C" int cdn_warp_affine_u8_batch(const uint8_t* d_pool, const cdn_warp_desc* h_desc, int n, uint8_t* d_dst, int dst_slots,
+                                        int dst_h, int dst_w, cdn_stream_t stream) {
+  CDN_CHECK(d_pool && h_desc && d_dst, CDN_ERR_INVALID, "warp_affine_batch: null pointer");
+  if (int rc = warp_batch_check("warp_affine_batch", h_desc, n, dst_slots, dst_h, dst_w)) return rc;
+  const int groups = (dst_w + WARP_PX - 1) / WARP_PX;
+  const long long tiles = ((long long)dst_h * groups + WARP_THREADS - 1) / WARP_THREADS;
   WarpBatchParams p;
   p.pool = d_pool; p.dst = d_dst; p.dh = dst_h; p.dw = dst_w; p.groups = groups; p.pad = 0;
   for (int base = 0; base < n; base += WARP_MAX_DESC) {
     const int m = std::min(WARP_MAX_DESC, n - base);
-    for (int i = 0; i < m; ++i) {
-      const cdn_warp_desc& d = h_desc[base + i];
-      WarpDesc& q = p.d[i];
-      q.off = d.src_offset; q.H = d.src_h; q.W = d.src_w; q.dst = d.dst_slot; q.mirror = d.mirror_slot;
-      warp_invert(d.M, q.m);
-    }
+    for (int i = 0; i < m; ++i) warp_fill(h_desc[base + i], p.d[i]);
     warp_affine_u8_kernel<<<dim3((unsigned)tiles, (unsigned)m), WARP_THREADS, 0, (cudaStream_t)stream>>>(p);
     CDN_LAUNCH_CHECK("warp_affine_u8_kernel");
+  }
+  return 0;
+}
+
+extern "C" int cdn_warp_affine_u8_f32_batch(const uint8_t* d_pool, const cdn_warp_desc* h_desc, const int32_t* h_table, int n,
+                                            const float* d_tables, int n_tables, float* d_dst, int dst_slots, int dst_h, int dst_w,
+                                            cdn_stream_t stream) {
+  CDN_CHECK(d_pool && h_desc && h_table && d_tables && d_dst, CDN_ERR_INVALID, "warp_affine_f32_batch: null pointer");
+  CDN_CHECK(((uintptr_t)d_tables & 3) == 0 && ((uintptr_t)d_dst & 3) == 0, CDN_ERR_INVALID,
+            "warp_affine_f32_batch: tables and destination must be 4-byte aligned");
+  CDN_CHECK(n_tables >= 1 && n_tables <= 2, CDN_ERR_INVALID, "warp_affine_f32_batch: n_tables = %d outside [1, 2]", n_tables);
+  if (int rc = warp_batch_check("warp_affine_f32_batch", h_desc, n, dst_slots, dst_h, dst_w)) return rc;
+  for (int i = 0; i < n; ++i)
+    CDN_CHECK(h_table[i] >= 0 && h_table[i] < n_tables, CDN_ERR_INVALID, "warp_affine_f32_batch: descriptor %d: table %d outside [0, %d)",
+              i, h_table[i], n_tables);
+  const int groups = (dst_w + WARP_PX - 1) / WARP_PX;
+  const long long tiles = ((long long)dst_h * groups + WARP_THREADS - 1) / WARP_THREADS;
+  WarpF32Params p;
+  p.pool = d_pool; p.dst = d_dst; p.tables = d_tables; p.dh = dst_h; p.dw = dst_w; p.groups = groups;
+  p.vec = dst_w % WARP_PX == 0 && ((uintptr_t)d_dst & 15) == 0;
+  for (int base = 0; base < n; base += WARP_F32_MAX_DESC) {
+    const int m = std::min(WARP_F32_MAX_DESC, n - base);
+    for (int i = 0; i < m; ++i) {
+      warp_fill(h_desc[base + i], p.d[i]);
+      p.table[i] = (uint8_t)h_table[base + i];
+    }
+    warp_affine_u8_f32_kernel<<<dim3((unsigned)tiles, (unsigned)m), WARP_THREADS, 0, (cudaStream_t)stream>>>(p);
+    CDN_LAUNCH_CHECK("warp_affine_u8_f32_kernel");
   }
   return 0;
 }

@@ -149,6 +149,19 @@ typedef struct cdn_warp_desc {
 #define CDN_WARP_DESC_PER_LAUNCH 454
 int cdn_warp_affine_u8_batch(const uint8_t* d_pool, const cdn_warp_desc* h_desc, int n, uint8_t* d_dst, int dst_slots, int dst_h,
                              int dst_w, cdn_stream_t stream);
+
+/* cdn_warp_affine_u8_f32_batch: the same ragged warp for the unquantised model, normalised into fp32 NCHW.  d_pool and h_desc as
+ * for cdn_warp_affine_u8_batch; d_tables is a device array [n_tables][3][256] fp32 (n_tables 1 or 2) and h_table[n] a HOST
+ * array with the table index of every descriptor.  Element (slot, c, y, x) of d_dst [dst_slots][3][dst_h][dst_w] is
+ * table[h_table[i]][c][v], v the byte cdn_warp_affine_u8_batch writes at (slot, y, x, c), mirror slot included; channels keep
+ * the frame's order.  The checks of cdn_warp_affine_u8_batch plus the tables pointer, n_tables and every table index, all on
+ * the host before anything is launched; d_tables and d_dst 4-byte aligned (float4 stores when dst_w % 4 == 0 and d_dst is
+ * 16-byte aligned).  No workspace, allocation or synchronisation: the call can be captured.  Up to
+ * CDN_WARP_F32_DESC_PER_LAUNCH descriptors per launch. */
+#define CDN_WARP_F32_DESC_PER_LAUNCH 448
+int cdn_warp_affine_u8_f32_batch(const uint8_t* d_pool, const cdn_warp_desc* h_desc, const int32_t* h_table, int n,
+                                 const float* d_tables, int n_tables, float* d_dst, int dst_slots, int dst_h, int dst_w,
+                                 cdn_stream_t stream);
 int cdn_ctdet_group_by_class(const float* d_dets, int batch, int K, int num_classes, float* d_out, int32_t* d_counts,
                              cdn_stream_t stream);
 
