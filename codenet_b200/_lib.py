@@ -42,6 +42,14 @@ WARP_DESC = np.dtype([("src_offset", np.int64), ("src_h", np.int32), ("src_w", n
 assert WARP_DESC.itemsize == 72
 WARP_DESC_PER_LAUNCH = 454         # CDN_WARP_DESC_PER_LAUNCH
 WARP_F32_DESC_PER_LAUNCH = 448     # CDN_WARP_F32_DESC_PER_LAUNCH (cdn_warp_affine_u8_f32_batch)
+# cdn_warp_src_desc: one output image of cdn_warp_affine_src_u8[_f32]_batch, its source frame given by device plane addresses
+WARP_SRC_DESC = np.dtype([("plane", np.uint64, (3,)), ("pitch", np.int64, (2,)), ("kind", np.int32), ("chroma_step", np.int32),
+                          ("src_h", np.int32), ("src_w", np.int32), ("M", np.float64, (6,)), ("dst_slot", np.int32),
+                          ("mirror_slot", np.int32)])
+assert WARP_SRC_DESC.itemsize == 112
+WARP_SRC_BGR, WARP_SRC_YUV420 = 0, 1               # CDN_WARP_SRC_BGR, CDN_WARP_SRC_YUV420
+WARP_SRC_DESC_PER_LAUNCH = 292     # CDN_WARP_SRC_DESC_PER_LAUNCH
+WARP_SRC_F32_DESC_PER_LAUNCH = 289  # CDN_WARP_SRC_F32_DESC_PER_LAUNCH
 
 EXPORTS = {
     "cdn_last_error": (C.c_char_p, []),
@@ -122,6 +130,9 @@ EXPORTS = {
     "cdn_warp_affine_u8_batch": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int, C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_void_p]),
     "cdn_warp_affine_u8_f32_batch": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.c_void_p, C.c_int, C.c_void_p, C.c_int,
                                                C.c_int, C.c_int, C.c_void_p]),
+    "cdn_warp_affine_src_u8_batch": (C.c_int, [C.c_void_p, C.c_int, C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_void_p]),
+    "cdn_warp_affine_src_u8_f32_batch": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int, C.c_void_p, C.c_int, C.c_void_p, C.c_int, C.c_int,
+                                                   C.c_int, C.c_void_p]),
     "cdn_jpeg_parse": (C.c_int, [C.c_void_p, C.c_int64, C.c_void_p]),
     "cdn_jpeg_decode_batch": (C.c_int, [C.c_void_p, C.c_int64, C.c_void_p, C.c_void_p, C.c_int, C.c_void_p, C.c_int64, C.c_void_p,
                                         C.c_int64, C.c_void_p, C.c_void_p]),

@@ -6,7 +6,8 @@ dict as the reference (`results` keyed by 1-based class id and the stage timers 
 Only what differs from the reference lives here: engine construction, process / process_u8, the device-side box transform,
 run()'s multi-scale path (all test scales of an image in one engine batch, merge_outputs on the device: cdn_ctdet_merge) and
 run_batch() (many raw frames per engine step, their warpAffine in one cdn_warp_affine_u8_batch launch per step, or for the
-unquantised model one cdn_warp_affine_u8_f32_batch launch that also normalises).
+unquantised model one cdn_warp_affine_u8_f32_batch launch that also normalises; the cdn_warp_affine_src_* forms when a step holds
+CUDA or YUV 4:2:0 frames).
 pre_process, merge_outputs and run keep the reference's contract (same inputs, outputs and timer keys) in this package's own
 decomposition (input_geometry / _Stages / group_by_class); INTEGRATION.md section 2 shows the patch for users who keep the reference's BaseDetector.
 """
@@ -16,6 +17,7 @@ from types import SimpleNamespace
 import numpy as np
 import torch
 
+from ..frames import YUV420, to_bgr
 from .nms import soft_nms
 from .decode import ctdet_decode
 from .quantize_model import quantize_shufflenetv2_dcn, freeze_ranges
@@ -459,6 +461,47 @@ class CtdetDetector:
             C.c_void_p(pool.data_ptr()), C.c_void_p(desc.ctypes.data), C.c_void_p(table.ctypes.data), len(desc),
             C.c_void_p(tables.data_ptr()), tables.shape[0], C.c_void_p(dst.data_ptr()), dst.shape[0], dst.shape[2], dst.shape[3], st))
 
+    def _warp_src(self, desc, dst):
+        """cdn_warp_affine_src_u8_batch on the current stream: the descriptors `desc` (_lib.WARP_SRC_DESC) into the uint8 CUDA batch
+        dst [slots, H, W, 3]."""
+        import ctypes as C
+        from .. import _lib
+        st = C.c_void_p(torch.cuda.current_stream(dst.device).cuda_stream)
+        _lib.check(_lib.load().cdn_warp_affine_src_u8_batch(C.c_void_p(desc.ctypes.data), len(desc), C.c_void_p(dst.data_ptr()),
+                                                             dst.shape[0], dst.shape[1], dst.shape[2], st))
+
+    def _warp_src_f32(self, desc, table, tables, dst):
+        """cdn_warp_affine_src_u8_f32_batch on the current stream: _warp_f32 with general-source descriptors (_lib.WARP_SRC_DESC)."""
+        import ctypes as C
+        from .. import _lib
+        st = C.c_void_p(torch.cuda.current_stream(dst.device).cuda_stream)
+        table = np.ascontiguousarray(table, dtype=np.int32)
+        _lib.check(_lib.load().cdn_warp_affine_src_u8_f32_batch(
+            C.c_void_p(desc.ctypes.data), C.c_void_p(table.ctypes.data), len(desc), C.c_void_p(tables.data_ptr()), tables.shape[0],
+            C.c_void_p(dst.data_ptr()), dst.shape[0], dst.shape[2], dst.shape[3], st))
+
+    def _frame_src_descs(self, frame, layout, host, pool, offsets, desc, slot0):
+        """Fills the general-source descriptors of every (scale 1) test scale of a CUDA BGR tensor or a YUV420 frame: slot0 + k for
+        scale k, or slot0 + 2k with the --flip_test mirror in slot0 + 2k + 1 (_pack_frame's slots).  CUDA planes are read where they
+        are; the planes of a host YUV420 frame are copied into the staging buffer `host` at `offsets` (Y, U, V, 1.5 bytes per
+        pixel), which the step's copy brings to the device pool `pool`."""
+        from .._lib import WARP_SRC_BGR, WARP_SRC_YUV420
+        n = 2 if self.opt.flip_test else 1
+        if isinstance(frame, torch.Tensor):
+            planes, pitch, kind, step = (frame.data_ptr(), 0, 0), (frame.stride(0), 0), WARP_SRC_BGR, 1
+        elif frame.is_cuda:
+            planes = tuple(p.data_ptr() for p in (frame.y, frame.u, frame.v))
+            pitch, kind, step = (frame.y.stride(0), frame.u.stride(0)), WARP_SRC_YUV420, frame.u.stride(1)
+        else:
+            for p, off in zip((frame.y, frame.u, frame.v), offsets):
+                host[off:off + p.size].reshape(p.shape)[...] = p
+            H, W = frame.shape
+            planes = tuple(pool.data_ptr() + off for off in offsets)
+            pitch, kind, step = (W, W // 2), WARP_SRC_YUV420, 1
+        for k, (sh, sw, M, _) in enumerate(layout):
+            slot = slot0 + n * k
+            desc[k] = (planes, pitch, kind, step, sh, sw, np.asarray(M, np.float64).reshape(6), slot, slot + 1 if n == 2 else -1)
+
     def _slots_u8(self, image, scales, ih, iw):
         """The network images of `scales` of one uint8 HWC frame as one uint8 CUDA batch [slots, ih, iw, 3] (scale-major, the
         mirror after its image): the frame and its host cv2.resize copies (scales other than 1) go to the device in one byte pool
@@ -606,7 +649,18 @@ class CtdetDetector:
         all frames and one copy back (_merge_on_device), which also brings the decode status of every device-decoded frame:
         a frame the device flagged (corrupt data) is decoded by cv2 and re-run through run().
         Needs fix_res (the engine is compiled for one input size; run() is the path for keep_res); prefetched dicts go through
-        run().  JPEGs of the unquantised model are decoded by cv2 on the host."""
+        run().  JPEGs of the unquantised model are decoded by cv2 on the host.
+
+        Frames may also be uint8 (H, W, 3) BGR CUDA tensors on the detector's device with strides (row >= 3W, 3, 1), e.g. crops of
+        a larger tensor, and YUV420 frames (codenet_b200.frames; host or device planes, I420 / YV12 / NV12 / NV21 views of a
+        decoder's surface).  Element i's results are run(t.cpu().numpy())'s for a tensor and run(to_bgr(f))'s for a YUV420 frame.
+        When every test scale is 1, a step holding any of them writes all its slots with one cdn_warp_affine_src_u8_batch (or, for
+        the unquantised model, cdn_warp_affine_src_u8_f32_batch) launch: CUDA planes are read in place, with none of their bytes
+        staged, host YUV420 planes are staged at 1.5 bytes per pixel and converted to BGR tap by tap inside the warp, and the
+        step's host arrays and device-decoded JPEGs are read from the pool as usual.  At other scale lists they take the host
+        path (one device -> host copy per CUDA frame, to_bgr per YUV420 frame, then the host cv2.resize): correct, not fast.
+        CUDA frames are read on the current stream of the detector's device, after the work already queued there: a frame
+        produced on another stream must be synchronised with it by the caller.  They may be freed once run_batch returns."""
         from .. import jpeg
         clock = _Stages()
         items = self._batch_frames(frames)
@@ -617,15 +671,13 @@ class CtdetDetector:
         n = 2 if opt.flip_test else 1
         S, F, ih, iw = len(self.scales), len(items), opt.input_h, opt.input_w
         spf = n * S
-        shapes = [im.shape[:2] if im is not None else (int(d[0]["height"]), int(d[0]["width"])) for im, _, d in items]
+        shapes = [_item_shape(item) for item in items]
         layouts = [self._frame_layout(h, w, self.scales) for h, w in shapes]
         metas = [m for layout in layouts for _, _, _, m in layout]
         max_batch = getattr(opt, "max_batch", 1)
-        # a JPEG stream is staged after the raw sources of its step (device decoding implies one test scale)
-        steps = plan_frame_steps([[0] if items[f][0] is None else [sh * sw * 3 for sh, sw, _, _ in layouts[f]] for f in range(F)],
-                                 spf, max_batch)
+        steps = plan_frame_steps([_staged_sources(items[f], layouts[f]) for f in range(F)], spf, max_batch)
         step_slots = max(int(max_batch), spf)
-        on_dev = [f for f in range(F) if items[f][0] is None]
+        on_dev = [f for f in range(F) if items[f][1] is not None]
         rank = {f: k for k, f in enumerate(on_dev)}
         from .._lib import WARP_DESC
         with torch.cuda.device(dev):
@@ -640,7 +692,8 @@ class CtdetDetector:
                 b = i % 2
                 if h2d_done[b] is not None:
                     h2d_done[b].synchronize()                  # staging buffer b is free again
-                jf = [f for f in fr if items[f][0] is None]
+                jf = [f for f in fr if items[f][1] is not None]
+                direct = [k for k, f in enumerate(fr) if _is_frame(items[f][2])]
                 staged = pool_bytes = nbytes
                 if jf:
                     # staged: raw sources, the descriptor table, the streams; the device pool goes on with the decoded frames
@@ -650,14 +703,15 @@ class CtdetDetector:
                     out_base = -(-staged // jpeg.WS_ALIGN) * jpeg.WS_ALIGN
                     desc["out_offset"] += out_base
                     pool_bytes = out_base + out_end
-                stage, pool, grown = self._staging(st, b, staged, pool_bytes)
-                host = stage.numpy()
-                wdesc = np.empty(len(fr) * S, WARP_DESC)
+                # a step of CUDA frames only stages nothing: they are read in place
+                stage, pool, grown = self._staging(st, b, staged, pool_bytes) if staged else (None, None, False)
+                host = stage.numpy() if staged else None
+                wdesc = np.zeros(len(fr) * S, WARP_DESC)
                 for k, f in enumerate(fr):
                     image, data, _ = items[f]
                     if image is not None:
                         self._pack_frame(image, layouts[f], self.scales, host, offsets[k], wdesc[k * S:(k + 1) * S], k * spf)
-                    else:
+                    elif data is not None:
                         j = jf.index(f)
                         host[soffs[j]:soffs[j] + data.size] = data
                         (sh, sw, M, _), = layouts[f]
@@ -665,23 +719,37 @@ class CtdetDetector:
                                     k * spf + 1 if n == 2 else -1)
                 if jf:
                     host[table:table + desc.nbytes] = desc.view(np.uint8)
-                if grown:
-                    # a new pool may reuse memory the compute stream freed with work still queued (e.g. the flip merge's maps)
-                    copy.wait_stream(compute)
-                elif warp_done[b] is not None:
-                    copy.wait_event(warp_done[b])              # the warp of step i - 2 has read device pool b
-                with torch.cuda.stream(copy):
-                    pool[:staged].copy_(stage[:staged], non_blocking=True)
-                    h2d_done[b] = torch.cuda.Event()
-                    h2d_done[b].record(copy)
-                compute.wait_event(h2d_done[b])
+                sdesc = None
+                if direct:
+                    # one general-source launch writes every slot of the step: the pool's frames as pitched BGR descriptors
+                    sdesc = _pool_src_descs(wdesc, pool)
+                    for k in direct:
+                        f = fr[k]
+                        self._frame_src_descs(items[f][2], layouts[f], host, pool, offsets[k], sdesc[k * S:(k + 1) * S], k * spf)
+                if staged:
+                    if grown:
+                        # a new pool may reuse memory the compute stream freed with work still queued (e.g. the flip merge's maps)
+                        copy.wait_stream(compute)
+                    elif warp_done[b] is not None:
+                        copy.wait_event(warp_done[b])              # the warp of step i - 2 has read device pool b
+                    with torch.cuda.stream(copy):
+                        pool[:staged].copy_(stage[:staged], non_blocking=True)
+                        h2d_done[b] = torch.cuda.Event()
+                        h2d_done[b].record(copy)
+                    compute.wait_event(h2d_done[b])
                 B = len(fr) * spf
                 if jf:
                     ws = self._jpeg_workspace(st, ws_bytes)
                     jpeg.decode_batch(pool.data_ptr(), pool.numel(), desc, pool.data_ptr() + table, ws.data_ptr(), ws.numel(),
                                       pool.data_ptr(), pool.numel(), status[rank[jf[0]]:].data_ptr(), compute.cuda_stream)
                 if self.float_model:
-                    self._warp_f32(pool, wdesc, self._table_index(self.scales, len(fr)), st["tables"], st["dst"])
+                    table_index = self._table_index(self.scales, len(fr))
+                    if direct:
+                        self._warp_src_f32(sdesc, table_index, st["tables"], st["dst"])
+                    else:
+                        self._warp_f32(pool, wdesc, table_index, st["tables"], st["dst"])
+                elif direct:
+                    self._warp_src(sdesc, st["dst"])
                 else:
                     self._warp(pool, wdesc, st["dst"])
                 warp_done[b] = torch.cuda.Event()
@@ -720,19 +788,31 @@ class CtdetDetector:
                 if f.dtype != np.uint8 or not (f.ndim == 1 or (f.ndim == 3 and f.shape[2] == 3)):
                     raise ValueError("run_batch takes uint8 HWC 3-channel frames or 1-D uint8 encoded images, got %s %s"
                                      % (f.dtype, f.shape))
+            elif isinstance(f, torch.Tensor):
+                self._check_cuda_frame(f)
+            elif isinstance(f, YUV420):
+                if f.is_cuda and f.y.device != self.opt.device:
+                    raise ValueError("run_batch: YUV420 planes on %s, the detector runs on %s" % (f.y.device, self.opt.device))
             elif not isinstance(f, (str, bytes, bytearray, memoryview)):
-                raise ValueError("run_batch takes uint8 arrays, image paths or encoded images, not %s (prefetched dicts go "
-                                 "through run())" % type(f).__name__)
+                raise ValueError("run_batch takes uint8 arrays, CUDA uint8 tensors, YUV420 frames, image paths or encoded images, not "
+                                 "%s (prefetched dicts go through run())" % type(f).__name__)
         # one restart interval decodes serially in one thread, so a device decode call costs about one frame's entropy decode
         # (13-41 ms for 500x375 q75-q95 on a B200) whatever the number of frames: it pays from JPEG_DEVICE_MIN_FRAMES per step
         spf = len(self.opt.test_scales) * (2 if self.opt.flip_test else 1)
         per_step = max(int(getattr(self.opt, "max_batch", 1)), spf) // spf
         device_jpeg = (self.opt.resume_quantize and list(self.opt.test_scales) == [1] and
                        min(per_step, len(frames)) >= JPEG_DEVICE_MIN_FRAMES)
+        # CUDA and YUV420 frames go to the general-source warp when every test scale is 1; otherwise pre_process's host cv2.resize
+        # needs them as host BGR images (one device -> host copy per CUDA frame, to_bgr per YUV420 frame): correct, not fast
+        direct = all(s == 1 for s in self.opt.test_scales)
         items = []
         for f in frames:
             if isinstance(f, np.ndarray) and f.ndim == 3:
                 items.append((f, None, None))
+                continue
+            if _is_frame(f):
+                items.append((None, None, f) if direct else
+                             (f.cpu().numpy() if isinstance(f, torch.Tensor) else to_bgr(f), None, None))
                 continue
             if isinstance(f, str):
                 try:
@@ -752,6 +832,17 @@ class CtdetDetector:
             except ValueError:
                 raise ValueError("run_batch: cannot read image %s" % (repr(f) if isinstance(f, str) else "(%d bytes)" % data.size)) from None
         return items
+
+    def _check_cuda_frame(self, t):
+        """Raises ValueError unless t is a uint8 (H, W, 3) BGR CUDA tensor on the detector's device with strides (row >= 3W, 3, 1)."""
+        if not t.is_cuda:
+            raise ValueError("run_batch takes CUDA tensors only, not a %s tensor (host frames are numpy arrays)" % t.device)
+        if t.device != self.opt.device:
+            raise ValueError("run_batch: CUDA frame on %s, the detector runs on %s" % (t.device, self.opt.device))
+        if t.dtype != torch.uint8 or t.dim() != 3 or t.shape[2] != 3 or t.shape[0] == 0 or t.shape[1] == 0:
+            raise ValueError("run_batch takes uint8 (H, W, 3) CUDA tensors, got %s %s" % (t.dtype, tuple(t.shape)))
+        if t.stride(2) != 1 or t.stride(1) != 3 or t.stride(0) < 3 * t.shape[1]:
+            raise ValueError("run_batch: a CUDA frame needs strides (row >= 3W, 3, 1), got %s" % (t.stride(),))
 
     def _batch_state(self, dev, step_slots, ih, iw, eng):
         """run_batch's device buffers, kept between calls so the engine replays the same graphs: the warp's destination batch,
@@ -800,6 +891,46 @@ class CtdetDetector:
 
 
 _BYTES = np.arange(256, dtype=np.uint8)
+
+
+def _is_frame(x):
+    """A run_batch input the general-source warp reads: a CUDA BGR tensor or a YUV420 frame."""
+    return isinstance(x, (torch.Tensor, YUV420))
+
+
+def _item_shape(item):
+    """(height, width) of a _batch_frames item."""
+    image, data, x = item
+    if image is not None:
+        return image.shape[:2]
+    if data is not None:
+        return int(x[0]["height"]), int(x[0]["width"])
+    return tuple(int(v) for v in x.shape[:2])
+
+
+def _staged_sources(item, layout):
+    """The byte sizes of what run_batch stages for one _batch_frames item (plan_frame_steps' source_bytes): the source image of
+    every test scale of a host array, the Y, U and V planes of a host YUV420 frame; nothing for a CUDA frame, read in place, or a
+    device-decoded JPEG, whose stream is staged after the raw sources of its step."""
+    image, _, x = item
+    if image is not None:
+        return [sh * sw * 3 for sh, sw, _, _ in layout]
+    if isinstance(x, YUV420) and not x.is_cuda:
+        H, W = x.shape
+        return [H * W, H * W // 4, H * W // 4]
+    return [0]
+
+
+def _pool_src_descs(wdesc, pool):
+    """cdn_warp_desc entries (offsets into the device pool) as general-source BGR descriptors (_lib.WARP_SRC_DESC)."""
+    from .._lib import WARP_SRC_DESC, WARP_SRC_BGR
+    d = np.zeros(len(wdesc), WARP_SRC_DESC)
+    d["plane"][:, 0] = (pool.data_ptr() if pool is not None else 0) + wdesc["src_offset"]
+    d["pitch"][:, 0] = 3 * wdesc["src_w"]
+    d["kind"], d["chroma_step"] = WARP_SRC_BGR, 1
+    for k in ("src_h", "src_w", "M", "dst_slot", "mirror_slot"):
+        d[k] = wdesc[k]
+    return d
 MERGE_MAX_ROWS = 1024          # CDN_SOFT_NMS_MAX_LEN: test scales x K rows per image that cdn_ctdet_merge takes
 # frames per run_batch step from which JPEGs are decoded on the device rather than by cv2 on the host: on one B200 (1000 W) with
 # 500x375 4:2:0 files the device decode lost at 16 frames per step and at 32 frames at q95, and won from 64 frames per step

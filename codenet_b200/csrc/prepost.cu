@@ -10,6 +10,9 @@
 //     warped byte goes through a 3 x 256 fp32 table (the normalisation of BaseDetector.pre_process, :66-68, is a function of
 //     the byte and its channel) and is written in planes.  Both kernels call one interpolation function, so the fp32 output is
 //     the u8 kernel's output looked up, by construction.
+//   * cdn_warp_affine_src_u8_batch / cdn_warp_affine_src_u8_f32_batch -- the same two warps from frames anywhere in device memory
+//     (absolute plane addresses, row pitches): BGR, or YUV 4:2:0 (I420, YV12, NV12, NV21) converted to BGR tap by tap with
+//     OpenCV's COLOR_YUV2BGR_* arithmetic, so that each output is cv2.warpAffine(cv2.cvtColor(frame, COLOR_YUV2BGR_*), ...).
 //   * cdn_ctdet_group_by_class -- the per-class grouping of ctdet_post_process (lib/utils/post_process.py:86-103): detections
 //     [B][K][6] reordered by class (stable, i.e. by descending score inside a class) + per-class counts, so the host only
 //     slices views.
@@ -38,6 +41,22 @@ struct WarpF32Params {
 };
 static_assert(offsetof(WarpF32Params, d) == 40, "WarpF32Params header");
 static_assert(sizeof(WarpF32Params) <= 32764, "kernel parameters exceed 32764 bytes");
+// cdn_warp_src_desc on the device: absolute plane addresses, row pitches, the INVERSE matrix
+struct WarpSrcDesc { const uint8_t* p[3]; long long pitch[2]; double m[6]; int H, W, kind, step, dst, mirror; };
+static_assert(sizeof(WarpSrcDesc) == 112, "WarpSrcDesc layout");
+static_assert(sizeof(cdn_warp_src_desc) == 112, "cdn_warp_src_desc layout (codenet_b200._lib.WARP_SRC_DESC)");
+// the general-source variants: 24 (u8) and 32 (fp32: 289 table bytes follow the descriptors) bytes of header
+constexpr int WARP_SRC_MAX_DESC = (32764 - 24) / (int)sizeof(WarpSrcDesc);
+static_assert(WARP_SRC_MAX_DESC == CDN_WARP_SRC_DESC_PER_LAUNCH, "include/codenet_b200.h states the descriptors per launch");
+struct WarpSrcParams { uint8_t* dst; int dh, dw, groups, pad; WarpSrcDesc d[WARP_SRC_MAX_DESC]; };
+static_assert(offsetof(WarpSrcParams, d) == 24 && sizeof(WarpSrcParams) <= 32764, "WarpSrcParams");
+constexpr int WARP_SRC_F32_MAX_DESC = (32764 - 32) / (int)(sizeof(WarpSrcDesc) + sizeof(uint8_t));
+static_assert(WARP_SRC_F32_MAX_DESC == CDN_WARP_SRC_F32_DESC_PER_LAUNCH, "include/codenet_b200.h states the descriptors per launch");
+struct WarpSrcF32Params {
+  float* dst; const float* tables; int dh, dw, groups, vec;
+  WarpSrcDesc d[WARP_SRC_F32_MAX_DESC]; uint8_t table[WARP_SRC_F32_MAX_DESC];
+};
+static_assert(offsetof(WarpSrcF32Params, d) == 32 && sizeof(WarpSrcF32Params) <= 32764, "WarpSrcF32Params");
 
 // cv::warpAffine's inversion of the 2 x 3 matrix (imgwarp.cpp), in double on the host: the same expressions on the device
 // would be contracted into FMAs and could round differently
@@ -65,11 +84,45 @@ __device__ __forceinline__ void warp_store(uint8_t* d, const uint8_t (&v)[WARP_P
   }
 }
 
+// How warp_pixels reads a tap: tap(yy, xx, w, acc) adds w x channel c (B, G, R) of source pixel (yy, xx), which lies inside the
+// frame, to acc[c].  PoolBgr: a uint8 BGR HWC frame of rows exactly 3W bytes long (cdn_warp_desc); PitchedBgr: the same with any row pitch;
+// Yuv420: Y, U and V planes of 4:2:0 video, converted per tap by OpenCV's COLOR_YUV2BGR_* (color_yuv.simd.hpp: BT.601 video
+// range, 20-bit fixed point), so that interpolating the converted taps is cv2.warpAffine(cv2.cvtColor(frame), ...) exactly.
+struct PoolBgr {
+  const uint8_t* src; const WarpDesc& q;
+  __device__ __forceinline__ void operator()(int yy, int xx, int w, int (&acc)[3]) const {
+    const uint8_t* s = src + ((size_t)yy * q.W + xx) * 3;
+#pragma unroll
+    for (int c = 0; c < 3; ++c) acc[c] += (int)__ldg(s + c) * w;
+  }
+};
+struct PitchedBgr {
+  const uint8_t* src; long long pitch;
+  __device__ __forceinline__ void operator()(int yy, int xx, int w, int (&acc)[3]) const {
+    const uint8_t* s = src + (size_t)yy * pitch + (size_t)xx * 3;
+#pragma unroll
+    for (int c = 0; c < 3; ++c) acc[c] += (int)__ldg(s + c) * w;
+  }
+};
+constexpr int YUV_CY = 1220542, YUV_CUB = 2116026, YUV_CUG = -409993, YUV_CVG = -852492, YUV_CVR = 1673527, YUV_SHIFT = 20;
+struct Yuv420 {
+  const uint8_t *y, *u, *v; long long pitch, chroma_pitch; int step;
+  __device__ __forceinline__ void operator()(int yy, int xx, int w, int (&acc)[3]) const {
+    const size_t c = (size_t)(yy >> 1) * chroma_pitch + (size_t)(xx >> 1) * step;
+    const int U = (int)__ldg(u + c) - 128, V = (int)__ldg(v + c) - 128;
+    // |each sum| < 2^30: int32 is exact, and >> is the arithmetic shift OpenCV's int arithmetic uses
+    const int l = max((int)__ldg(y + (size_t)yy * pitch + xx) - 16, 0) * YUV_CY + (1 << (YUV_SHIFT - 1));
+    acc[0] += min(max((l + YUV_CUB * U) >> YUV_SHIFT, 0), 255) * w;
+    acc[1] += min(max((l + YUV_CVG * V + YUV_CUG * U) >> YUV_SHIFT, 0), 255) * w;
+    acc[2] += min(max((l + YUV_CVR * V) >> YUV_SHIFT, 0), 255) * w;
+  }
+};
+
 // OpenCV's fixed-point bilinear interpolation of WARP_PX consecutive destination pixels (y, x0 .. x0 + WARP_PX - 1) of one
-// descriptor, the one both warp kernels call: v[i * 3 + c] = channel c of pixel x0 + i (a pixel past the row's end is
-// computed like the others and left unstored by the caller)
-__device__ __forceinline__ void warp_pixels(const WarpDesc& q, const uint8_t* pool, int y, int x0, uint8_t (&v)[WARP_PX * 3]) {
-  const uint8_t* src = pool + q.off;
+// H x W source through the inverse matrix m, the one every warp kernel calls: v[i * 3 + c] = channel c of pixel x0 + i (a pixel
+// past the row's end is computed like the others and left unstored by the caller).  Tap reads a source pixel (PoolBgr, ...).
+template <class Desc, class Tap>
+__device__ __forceinline__ void warp_pixels(const Desc& q, const Tap& tap3, int y, int x0, uint8_t (&v)[WARP_PX * 3]) {
   // dst -> src map in 1/1024 pixel, as OpenCV forms it: per-column and per-row terms are rounded SEPARATELY, then summed;
   // the row term is m1 * y + m2 in two roundings (no FMA), like OpenCV's and numpy's double arithmetic
   const int X0 = __double2int_rn(__dmul_rn(__dadd_rn(__dmul_rn(q.m[1], (double)y), q.m[2]), 1024.0)) + 16;
@@ -85,11 +138,7 @@ __device__ __forceinline__ void warp_pixels(const WarpDesc& q, const uint8_t* po
     const int w00 = (32 - fy) * (32 - fx) * 32, w01 = (32 - fy) * fx * 32, w10 = fy * (32 - fx) * 32, w11 = fy * fx * 32;
     int acc[3] = {0, 0, 0};
     auto tap = [&](int yy, int xx, int w) {
-      if ((unsigned)yy < (unsigned)q.H && (unsigned)xx < (unsigned)q.W) {
-        const uint8_t* s = src + ((size_t)yy * q.W + xx) * 3;
-#pragma unroll
-        for (int c = 0; c < 3; ++c) acc[c] += (int)__ldg(s + c) * w;
-      }
+      if ((unsigned)yy < (unsigned)q.H && (unsigned)xx < (unsigned)q.W) tap3(yy, xx, w, acc);
     };
     tap(sy, sx, w00); tap(sy, sx + 1, w01); tap(sy + 1, sx, w10); tap(sy + 1, sx + 1, w11);
 #pragma unroll
@@ -105,7 +154,7 @@ __global__ void __launch_bounds__(WARP_THREADS) warp_affine_u8_kernel(const __gr
   if (y >= p.dh) return;
   const int n = min(WARP_PX, p.dw - x0);
   uint8_t v[WARP_PX * 3];
-  warp_pixels(q, p.pool, y, x0, v);
+  warp_pixels(q, PoolBgr{p.pool + q.off, q}, y, x0, v);
   const size_t plane = (size_t)p.dh * p.dw * 3, row = (size_t)y * p.dw * 3;
   warp_store(p.dst + (size_t)q.dst * plane + row + (size_t)x0 * 3, v, n);
   if (q.mirror >= 0) {                               // the n pixels reversed, ending at column dw - 1 - x0
@@ -140,7 +189,7 @@ __global__ void __launch_bounds__(WARP_THREADS) warp_affine_u8_f32_kernel(const 
   if (y >= p.dh) return;
   const int n = min(WARP_PX, p.dw - x0);
   uint8_t v[WARP_PX * 3];
-  warp_pixels(q, p.pool, y, x0, v);
+  warp_pixels(q, PoolBgr{p.pool + q.off, q}, y, x0, v);
   const size_t plane = (size_t)p.dh * p.dw, row = (size_t)y * p.dw;
   float* d = p.dst + (size_t)q.dst * 3 * plane + row + x0;
   float* m = q.mirror >= 0 ? p.dst + (size_t)q.mirror * 3 * plane + row + (p.dw - x0 - n) : nullptr;   // ends at dw - 1 - x0
@@ -163,8 +212,80 @@ __global__ void __launch_bounds__(WARP_THREADS) warp_affine_u8_f32_kernel(const 
   }
 }
 
-// the checks both batch entry points make before anything is launched
-static int warp_batch_check(const char* who, const cdn_warp_desc* h_desc, int n, int dst_slots, int dst_h, int dst_w) {
+// The general-source kernels: the kernels above with each descriptor's frame read through its own tap, BGR at any row pitch or
+// YUV 4:2:0 (the source kind is uniform per CTA: blockIdx.y selects the descriptor).  The stores are those of the kernels above,
+// which keep their own code so that their SASS stays as it is.
+__device__ __forceinline__ void warp_src_pixels(const WarpSrcDesc& q, int y, int x0, uint8_t (&v)[WARP_PX * 3]) {
+  if (q.kind == CDN_WARP_SRC_YUV420)
+    warp_pixels(q, Yuv420{q.p[0], q.p[1], q.p[2], q.pitch[0], q.pitch[1], q.step}, y, x0, v);
+  else
+    warp_pixels(q, PitchedBgr{q.p[0], q.pitch[0]}, y, x0, v);
+}
+
+__global__ void __launch_bounds__(WARP_THREADS) warp_affine_src_u8_kernel(const __grid_constant__ WarpSrcParams p) {
+  const WarpSrcDesc& q = p.d[blockIdx.y];
+  const int t = blockIdx.x * WARP_THREADS + threadIdx.x;
+  const int y = t / p.groups, x0 = (t - y * p.groups) * WARP_PX;
+  if (y >= p.dh) return;
+  const int n = min(WARP_PX, p.dw - x0);
+  uint8_t v[WARP_PX * 3];
+  warp_src_pixels(q, y, x0, v);
+  const size_t plane = (size_t)p.dh * p.dw * 3, row = (size_t)y * p.dw * 3;
+  warp_store(p.dst + (size_t)q.dst * plane + row + (size_t)x0 * 3, v, n);
+  if (q.mirror >= 0) {
+    uint8_t f[WARP_PX * 3];
+#pragma unroll
+    for (int i = 0; i < WARP_PX; ++i)
+#pragma unroll
+      for (int c = 0; c < 3; ++c) f[i * 3 + c] = v[(WARP_PX - 1 - i) * 3 + c];
+    uint8_t* m = p.dst + (size_t)q.mirror * plane + row + (size_t)(p.dw - x0 - n) * 3;
+    if (n == WARP_PX) {
+      warp_store(m, f, n);
+    } else {
+      const int skip = (WARP_PX - n) * 3;
+#pragma unroll
+      for (int i = 0; i < WARP_PX * 3; ++i)
+        if (i >= skip) m[i - skip] = f[i];
+    }
+  }
+}
+
+__global__ void __launch_bounds__(WARP_THREADS) warp_affine_src_u8_f32_kernel(const __grid_constant__ WarpSrcF32Params p) {
+  __shared__ float s_tab[3 * 256];
+  const WarpSrcDesc& q = p.d[blockIdx.y];
+  const float* tab = p.tables + (size_t)p.table[blockIdx.y] * (3 * 256);
+  for (int i = threadIdx.x; i < 3 * 256; i += WARP_THREADS) s_tab[i] = __ldg(tab + i);
+  __syncthreads();
+  const int t = blockIdx.x * WARP_THREADS + threadIdx.x;
+  const int y = t / p.groups, x0 = (t - y * p.groups) * WARP_PX;
+  if (y >= p.dh) return;
+  const int n = min(WARP_PX, p.dw - x0);
+  uint8_t v[WARP_PX * 3];
+  warp_src_pixels(q, y, x0, v);
+  const size_t plane = (size_t)p.dh * p.dw, row = (size_t)y * p.dw;
+  float* d = p.dst + (size_t)q.dst * 3 * plane + row + x0;
+  float* m = q.mirror >= 0 ? p.dst + (size_t)q.mirror * 3 * plane + row + (p.dw - x0 - n) : nullptr;
+#pragma unroll
+  for (int c = 0; c < 3; ++c) {
+    float f[WARP_PX];
+#pragma unroll
+    for (int i = 0; i < WARP_PX; ++i) f[i] = s_tab[c * 256 + v[i * 3 + c]];
+    if (p.vec) {
+      *reinterpret_cast<float4*>(d + c * plane) = make_float4(f[0], f[1], f[2], f[3]);
+      if (m) *reinterpret_cast<float4*>(m + c * plane) = make_float4(f[3], f[2], f[1], f[0]);
+    } else {
+#pragma unroll
+      for (int i = 0; i < WARP_PX; ++i)
+        if (i < n) {
+          d[c * plane + i] = f[i];
+          if (m) m[c * plane + n - 1 - i] = f[i];
+        }
+    }
+  }
+}
+
+// the destination checks of every batch entry point
+static int warp_dst_check(const char* who, int n, int dst_slots, int dst_h, int dst_w) {
   CDN_CHECK(n >= 0, CDN_ERR_INVALID, "%s: n = %d", who, n);
   CDN_CHECK(dst_slots > 0 && dst_h > 0 && dst_w > 0, CDN_ERR_INVALID, "%s: bad destination %d x %d x %d", who, dst_slots, dst_h,
             dst_w);
@@ -172,6 +293,12 @@ static int warp_batch_check(const char* who, const cdn_warp_desc* h_desc, int n,
   const long long tiles = ((long long)dst_h * groups + WARP_THREADS - 1) / WARP_THREADS;
   CDN_CHECK(tiles <= 0x7fffffffLL && (long long)dst_h * groups <= 0x7fffffffLL, CDN_ERR_INVALID,
             "%s: destination %d x %d too large", who, dst_h, dst_w);
+  return 0;
+}
+
+// the checks both pool batch entry points make before anything is launched
+static int warp_batch_check(const char* who, const cdn_warp_desc* h_desc, int n, int dst_slots, int dst_h, int dst_w) {
+  if (int rc = warp_dst_check(who, n, dst_slots, dst_h, dst_w)) return rc;
   for (int i = 0; i < n; ++i) {
     const cdn_warp_desc& d = h_desc[i];
     CDN_CHECK(d.src_offset >= 0 && d.src_h > 0 && d.src_w > 0, CDN_ERR_INVALID,
@@ -182,8 +309,44 @@ static int warp_batch_check(const char* who, const cdn_warp_desc* h_desc, int n,
   return 0;
 }
 
+// the checks both general-source entry points make before anything is launched: what every plane must hold, per source kind
+static int warp_src_check(const char* who, const cdn_warp_src_desc* h_desc, int n, int dst_slots, int dst_h, int dst_w) {
+  if (int rc = warp_dst_check(who, n, dst_slots, dst_h, dst_w)) return rc;
+  for (int i = 0; i < n; ++i) {
+    const cdn_warp_src_desc& d = h_desc[i];
+    CDN_CHECK(d.kind == CDN_WARP_SRC_BGR || d.kind == CDN_WARP_SRC_YUV420, CDN_ERR_INVALID, "%s: descriptor %d: unknown source kind %d",
+              who, i, d.kind);
+    CDN_CHECK(d.src_h > 0 && d.src_w > 0, CDN_ERR_INVALID, "%s: descriptor %d: bad source size %d x %d", who, i, d.src_h, d.src_w);
+    if (d.kind == CDN_WARP_SRC_BGR) {
+      CDN_CHECK(d.plane[0], CDN_ERR_INVALID, "%s: descriptor %d: null plane", who, i);
+      CDN_CHECK(d.pitch[0] >= 3LL * d.src_w, CDN_ERR_INVALID, "%s: descriptor %d: pitch %lld below the row's %lld bytes", who, i,
+                d.pitch[0], 3LL * d.src_w);
+    } else {
+      CDN_CHECK(d.plane[0] && d.plane[1] && d.plane[2], CDN_ERR_INVALID, "%s: descriptor %d: null plane", who, i);
+      CDN_CHECK(d.src_h % 2 == 0 && d.src_w % 2 == 0, CDN_ERR_INVALID, "%s: descriptor %d: odd YUV 4:2:0 size %d x %d", who, i,
+                d.src_h, d.src_w);
+      CDN_CHECK(d.chroma_step == 1 || d.chroma_step == 2, CDN_ERR_INVALID, "%s: descriptor %d: chroma step %d not 1 or 2", who, i,
+                d.chroma_step);
+      const long long chroma_row = (long long)(d.src_w / 2 - 1) * d.chroma_step + 1;
+      CDN_CHECK(d.pitch[0] >= d.src_w && d.pitch[1] >= chroma_row, CDN_ERR_INVALID,
+                "%s: descriptor %d: pitch %lld / %lld below the rows' %d / %lld bytes", who, i, d.pitch[0], d.pitch[1], d.src_w,
+                chroma_row);
+    }
+    CDN_CHECK(d.dst_slot >= 0 && d.dst_slot < dst_slots && d.mirror_slot >= -1 && d.mirror_slot < dst_slots, CDN_ERR_INVALID,
+              "%s: descriptor %d: slot %d / mirror %d outside [0, %d)", who, i, d.dst_slot, d.mirror_slot, dst_slots);
+  }
+  return 0;
+}
+
 static void warp_fill(const cdn_warp_desc& d, WarpDesc& q) {
   q.off = d.src_offset; q.H = d.src_h; q.W = d.src_w; q.dst = d.dst_slot; q.mirror = d.mirror_slot;
+  warp_invert(d.M, q.m);
+}
+
+static void warp_src_fill(const cdn_warp_src_desc& d, WarpSrcDesc& q) {
+  for (int k = 0; k < 3; ++k) q.p[k] = d.plane[k];
+  q.pitch[0] = d.pitch[0]; q.pitch[1] = d.pitch[1];
+  q.H = d.src_h; q.W = d.src_w; q.kind = d.kind; q.step = d.chroma_step; q.dst = d.dst_slot; q.mirror = d.mirror_slot;
   warp_invert(d.M, q.m);
 }
 
@@ -228,6 +391,50 @@ extern "C" int cdn_warp_affine_u8_f32_batch(const uint8_t* d_pool, const cdn_war
     }
     warp_affine_u8_f32_kernel<<<dim3((unsigned)tiles, (unsigned)m), WARP_THREADS, 0, (cudaStream_t)stream>>>(p);
     CDN_LAUNCH_CHECK("warp_affine_u8_f32_kernel");
+  }
+  return 0;
+}
+
+extern "C" int cdn_warp_affine_src_u8_batch(const cdn_warp_src_desc* h_desc, int n, uint8_t* d_dst, int dst_slots, int dst_h,
+                                            int dst_w, cdn_stream_t stream) {
+  CDN_CHECK(h_desc && d_dst, CDN_ERR_INVALID, "warp_affine_src_batch: null pointer");
+  if (int rc = warp_src_check("warp_affine_src_batch", h_desc, n, dst_slots, dst_h, dst_w)) return rc;
+  const int groups = (dst_w + WARP_PX - 1) / WARP_PX;
+  const long long tiles = ((long long)dst_h * groups + WARP_THREADS - 1) / WARP_THREADS;
+  WarpSrcParams p;
+  p.dst = d_dst; p.dh = dst_h; p.dw = dst_w; p.groups = groups; p.pad = 0;
+  for (int base = 0; base < n; base += WARP_SRC_MAX_DESC) {
+    const int m = std::min(WARP_SRC_MAX_DESC, n - base);
+    for (int i = 0; i < m; ++i) warp_src_fill(h_desc[base + i], p.d[i]);
+    warp_affine_src_u8_kernel<<<dim3((unsigned)tiles, (unsigned)m), WARP_THREADS, 0, (cudaStream_t)stream>>>(p);
+    CDN_LAUNCH_CHECK("warp_affine_src_u8_kernel");
+  }
+  return 0;
+}
+
+extern "C" int cdn_warp_affine_src_u8_f32_batch(const cdn_warp_src_desc* h_desc, const int32_t* h_table, int n, const float* d_tables,
+                                                int n_tables, float* d_dst, int dst_slots, int dst_h, int dst_w, cdn_stream_t stream) {
+  CDN_CHECK(h_desc && h_table && d_tables && d_dst, CDN_ERR_INVALID, "warp_affine_src_f32_batch: null pointer");
+  CDN_CHECK(((uintptr_t)d_tables & 3) == 0 && ((uintptr_t)d_dst & 3) == 0, CDN_ERR_INVALID,
+            "warp_affine_src_f32_batch: tables and destination must be 4-byte aligned");
+  CDN_CHECK(n_tables >= 1 && n_tables <= 2, CDN_ERR_INVALID, "warp_affine_src_f32_batch: n_tables = %d outside [1, 2]", n_tables);
+  if (int rc = warp_src_check("warp_affine_src_f32_batch", h_desc, n, dst_slots, dst_h, dst_w)) return rc;
+  for (int i = 0; i < n; ++i)
+    CDN_CHECK(h_table[i] >= 0 && h_table[i] < n_tables, CDN_ERR_INVALID,
+              "warp_affine_src_f32_batch: descriptor %d: table %d outside [0, %d)", i, h_table[i], n_tables);
+  const int groups = (dst_w + WARP_PX - 1) / WARP_PX;
+  const long long tiles = ((long long)dst_h * groups + WARP_THREADS - 1) / WARP_THREADS;
+  WarpSrcF32Params p;
+  p.dst = d_dst; p.tables = d_tables; p.dh = dst_h; p.dw = dst_w; p.groups = groups;
+  p.vec = dst_w % WARP_PX == 0 && ((uintptr_t)d_dst & 15) == 0;
+  for (int base = 0; base < n; base += WARP_SRC_F32_MAX_DESC) {
+    const int m = std::min(WARP_SRC_F32_MAX_DESC, n - base);
+    for (int i = 0; i < m; ++i) {
+      warp_src_fill(h_desc[base + i], p.d[i]);
+      p.table[i] = (uint8_t)h_table[base + i];
+    }
+    warp_affine_src_u8_f32_kernel<<<dim3((unsigned)tiles, (unsigned)m), WARP_THREADS, 0, (cudaStream_t)stream>>>(p);
+    CDN_LAUNCH_CHECK("warp_affine_src_u8_f32_kernel");
   }
   return 0;
 }

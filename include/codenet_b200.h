@@ -162,6 +162,38 @@ int cdn_warp_affine_u8_batch(const uint8_t* d_pool, const cdn_warp_desc* h_desc,
 int cdn_warp_affine_u8_f32_batch(const uint8_t* d_pool, const cdn_warp_desc* h_desc, const int32_t* h_table, int n,
                                  const float* d_tables, int n_tables, float* d_dst, int dst_slots, int dst_h, int dst_w,
                                  cdn_stream_t stream);
+
+/* cdn_warp_affine_src_u8_batch / cdn_warp_affine_src_u8_f32_batch: cdn_warp_affine_u8_batch and cdn_warp_affine_u8_f32_batch
+ * (same destinations, tables, table indices, mirrors and host checks) from source frames anywhere in device memory: a staging
+ * pool, a caller's tensor, a pitched decoder surface.  Each cdn_warp_src_desc gives absolute device plane addresses and row
+ * pitches in bytes:
+ *   kind CDN_WARP_SRC_BGR: uint8 BGR HWC rows of src_w * 3 bytes at plane[0] + y * pitch[0] (pitch[0] >= 3 src_w); plane[1],
+ *     plane[2], pitch[1] and chroma_step are not read.
+ *   kind CDN_WARP_SRC_YUV420: 4:2:0 video, src_h and src_w even.  Y (src_w bytes a row) at plane[0] + y * pitch[0]; U and V
+ *     (src_w / 2 samples a row, chroma_step bytes apart) at plane[1|2] + (y / 2) * pitch[1] + (x / 2) * chroma_step, so I420 / YV12
+ *     are chroma_step 1 and NV12 / NV21 are chroma_step 2 with the two planes one byte apart.  Every tap is converted to BGR as
+ *     OpenCV's cv2.cvtColor(..., COLOR_YUV2BGR_I420 | _YV12 | _NV12 | _NV21) does (BT.601 video range in 20-bit fixed point), so
+ *     the output is cv2.warpAffine of the converted frame bit for bit.
+ * Rejected on the host before anything is launched, past the first launch's worth too: null pointers, n < 0, an unknown kind,
+ * non-positive or odd YUV sizes, a null plane the kind reads, chroma_step not 1 or 2, a pitch shorter than its row (3 src_w, src_w,
+ * (src_w / 2 - 1) * chroma_step + 1), slots or table indices out of range.  No workspace, allocation or synchronisation: the call
+ * can be captured.  Up to CDN_WARP_SRC[_F32]_DESC_PER_LAUNCH descriptors per launch. */
+#define CDN_WARP_SRC_BGR 0
+#define CDN_WARP_SRC_YUV420 1
+typedef struct cdn_warp_src_desc {
+  const uint8_t* plane[3];           /* device addresses: BGR plane[0]; YUV Y, U, V */
+  long long pitch[2];                /* row pitch in bytes of plane 0 and of the chroma planes */
+  int kind, chroma_step;             /* CDN_WARP_SRC_*; bytes between chroma samples of a row (1 or 2) */
+  int src_h, src_w;
+  double M[6];                       /* the 2x3 source -> destination matrix cv2.warpAffine receives, row major */
+  int dst_slot, mirror_slot;
+} cdn_warp_src_desc;
+#define CDN_WARP_SRC_DESC_PER_LAUNCH 292
+#define CDN_WARP_SRC_F32_DESC_PER_LAUNCH 289
+int cdn_warp_affine_src_u8_batch(const cdn_warp_src_desc* h_desc, int n, uint8_t* d_dst, int dst_slots, int dst_h, int dst_w,
+                                 cdn_stream_t stream);
+int cdn_warp_affine_src_u8_f32_batch(const cdn_warp_src_desc* h_desc, const int32_t* h_table, int n, const float* d_tables,
+                                     int n_tables, float* d_dst, int dst_slots, int dst_h, int dst_w, cdn_stream_t stream);
 int cdn_ctdet_group_by_class(const float* d_dets, int batch, int K, int num_classes, float* d_out, int32_t* d_counts,
                              cdn_stream_t stream);
 
