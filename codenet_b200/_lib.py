@@ -50,6 +50,13 @@ assert WARP_SRC_DESC.itemsize == 112
 WARP_SRC_BGR, WARP_SRC_YUV420 = 0, 1               # CDN_WARP_SRC_BGR, CDN_WARP_SRC_YUV420
 WARP_SRC_DESC_PER_LAUNCH = 292     # CDN_WARP_SRC_DESC_PER_LAUNCH
 WARP_SRC_F32_DESC_PER_LAUNCH = 289  # CDN_WARP_SRC_F32_DESC_PER_LAUNCH
+# cdn_warp_rs_desc: one output image of cdn_warp_affine_resize_u8[_f32]_batch, a src_h x src_w frame resized to rs_h x rs_w first
+WARP_RS_DESC = np.dtype([("plane", np.uint64, (3,)), ("pitch", np.int64, (2,)), ("kind", np.int32), ("chroma_step", np.int32),
+                         ("src_h", np.int32), ("src_w", np.int32), ("rs_h", np.int32), ("rs_w", np.int32),
+                         ("inv_scale", np.float64, (2,)), ("M", np.float64, (6,)), ("dst_slot", np.int32), ("mirror_slot", np.int32)])
+assert WARP_RS_DESC.itemsize == 136
+WARP_RS_DESC_PER_LAUNCH = 240       # CDN_WARP_RS_DESC_PER_LAUNCH
+WARP_RS_F32_DESC_PER_LAUNCH = 238   # CDN_WARP_RS_F32_DESC_PER_LAUNCH
 
 EXPORTS = {
     "cdn_last_error": (C.c_char_p, []),
@@ -133,6 +140,9 @@ EXPORTS = {
     "cdn_warp_affine_src_u8_batch": (C.c_int, [C.c_void_p, C.c_int, C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_void_p]),
     "cdn_warp_affine_src_u8_f32_batch": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int, C.c_void_p, C.c_int, C.c_void_p, C.c_int, C.c_int,
                                                    C.c_int, C.c_void_p]),
+    "cdn_warp_affine_resize_u8_batch": (C.c_int, [C.c_void_p, C.c_int, C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_void_p]),
+    "cdn_warp_affine_resize_u8_f32_batch": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int, C.c_void_p, C.c_int, C.c_void_p, C.c_int,
+                                                      C.c_int, C.c_int, C.c_void_p]),
     "cdn_jpeg_parse": (C.c_int, [C.c_void_p, C.c_int64, C.c_void_p]),
     "cdn_jpeg_decode_batch": (C.c_int, [C.c_void_p, C.c_int64, C.c_void_p, C.c_void_p, C.c_int, C.c_void_p, C.c_int64, C.c_void_p,
                                         C.c_int64, C.c_void_p, C.c_void_p]),

@@ -7,7 +7,8 @@ Only what differs from the reference lives here: engine construction, process / 
 run()'s multi-scale path (all test scales of an image in one engine batch, merge_outputs on the device: cdn_ctdet_merge) and
 run_batch() (many raw frames per engine step, their warpAffine in one cdn_warp_affine_u8_batch launch per step, or for the
 unquantised model one cdn_warp_affine_u8_f32_batch launch that also normalises; the cdn_warp_affine_src_* forms when a step holds
-CUDA or YUV 4:2:0 frames).
+CUDA or YUV 4:2:0 frames, the cdn_warp_affine_resize_* forms, which also resize, with opt.device_resize at scale lists other
+than [1]).
 pre_process, merge_outputs and run keep the reference's contract (same inputs, outputs and timer keys) in this package's own
 decomposition (input_geometry / _Stages / group_by_class); INTEGRATION.md section 2 shows the patch for users who keep the reference's BaseDetector.
 """
@@ -441,6 +442,15 @@ class CtdetDetector:
             slot = slot0 + n * k
             desc[k] = (off, sh, sw, np.asarray(M, np.float64).reshape(6), slot, slot + 1 if n == 2 else -1)
 
+    def _frame_descs(self, desc, off, shape, layout, slot0):
+        """Fills the cdn_warp_desc entries of every test scale of a frame held at 1x in the device pool at `off` (a host array staged
+        once, a device-decoded JPEG): source size the frame's own, slots as _pack_frame's.  _rs_descs then gives each its
+        scale's resized size."""
+        n = 2 if self.opt.flip_test else 1
+        for k, (_, _, M, _) in enumerate(layout):
+            slot = slot0 + n * k
+            desc[k] = (off, shape[0], shape[1], np.asarray(M, np.float64).reshape(6), slot, slot + 1 if n == 2 else -1)
+
     def _warp(self, pool, desc, dst):
         """cdn_warp_affine_u8_batch on the current stream: the descriptors `desc` (_lib.WARP_DESC) from the device byte pool into
         the uint8 CUDA batch dst [slots, H, W, 3]."""
@@ -463,25 +473,48 @@ class CtdetDetector:
 
     def _warp_src(self, desc, dst):
         """cdn_warp_affine_src_u8_batch on the current stream: the descriptors `desc` (_lib.WARP_SRC_DESC) into the uint8 CUDA batch
-        dst [slots, H, W, 3]."""
+        dst [slots, H, W, 3]; cdn_warp_affine_resize_u8_batch for resize descriptors (_lib.WARP_RS_DESC)."""
         import ctypes as C
         from .. import _lib
         st = C.c_void_p(torch.cuda.current_stream(dst.device).cuda_stream)
-        _lib.check(_lib.load().cdn_warp_affine_src_u8_batch(C.c_void_p(desc.ctypes.data), len(desc), C.c_void_p(dst.data_ptr()),
-                                                             dst.shape[0], dst.shape[1], dst.shape[2], st))
+        fn = _lib.load().cdn_warp_affine_resize_u8_batch if desc.dtype == _lib.WARP_RS_DESC else _lib.load().cdn_warp_affine_src_u8_batch
+        _lib.check(fn(C.c_void_p(desc.ctypes.data), len(desc), C.c_void_p(dst.data_ptr()), dst.shape[0], dst.shape[1], dst.shape[2], st))
 
     def _warp_src_f32(self, desc, table, tables, dst):
-        """cdn_warp_affine_src_u8_f32_batch on the current stream: _warp_f32 with general-source descriptors (_lib.WARP_SRC_DESC)."""
+        """cdn_warp_affine_src_u8_f32_batch on the current stream: _warp_f32 with general-source descriptors (_lib.WARP_SRC_DESC);
+        cdn_warp_affine_resize_u8_f32_batch for resize descriptors (_lib.WARP_RS_DESC)."""
         import ctypes as C
         from .. import _lib
         st = C.c_void_p(torch.cuda.current_stream(dst.device).cuda_stream)
         table = np.ascontiguousarray(table, dtype=np.int32)
-        _lib.check(_lib.load().cdn_warp_affine_src_u8_f32_batch(
+        L = _lib.load()
+        fn = L.cdn_warp_affine_resize_u8_f32_batch if desc.dtype == _lib.WARP_RS_DESC else L.cdn_warp_affine_src_u8_f32_batch
+        _lib.check(fn(
             C.c_void_p(desc.ctypes.data), C.c_void_p(table.ctypes.data), len(desc), C.c_void_p(tables.data_ptr()), tables.shape[0],
             C.c_void_p(dst.data_ptr()), dst.shape[0], dst.shape[2], dst.shape[3], st))
 
+    def _resize_exact(self, height, width):
+        """True when every test scale's cv2.resize of an height x width frame is one the device resize reproduces
+        (device_resize_exact)."""
+        return all(device_resize_exact(height, width, *self.input_geometry(height, width, s)[0]) for s in self.opt.test_scales)
+
+    def _device_resize(self):
+        """True when run_batch resizes on the device: opt.device_resize is set and a test scale is not 1.  It is off unless asked
+        for, so run_batch's default stays the host cv2.resize of pre_process at every scale list."""
+        return bool(getattr(self.opt, "device_resize", False)) and any(s != 1 for s in self.opt.test_scales)
+
+    def _resized_on_device(self, item):
+        """True when run_batch resizes a _batch_frames item inside the warp (cdn_warp_affine_resize_*): with _device_resize, host
+        arrays that _resize_exact accepts and every CUDA, YUV420 or device-decoded frame (_batch_frames keeps those only when it
+        accepts them)."""
+        if not self._device_resize():
+            return False
+        image = item[0]
+        return image is None or self._resize_exact(*image.shape[:2])
+
     def _frame_src_descs(self, frame, layout, host, pool, offsets, desc, slot0):
-        """Fills the general-source descriptors of every (scale 1) test scale of a CUDA BGR tensor or a YUV420 frame: slot0 + k for
+        """Fills the general-source descriptors of every test scale of a CUDA BGR tensor or a YUV420 frame, source size the frame's
+        own (_rs_descs gives each its scale's resized size): slot0 + k for
         scale k, or slot0 + 2k with the --flip_test mirror in slot0 + 2k + 1 (_pack_frame's slots).  CUDA planes are read where they
         are; the planes of a host YUV420 frame are copied into the staging buffer `host` at `offsets` (Y, U, V, 1.5 bytes per
         pixel), which the step's copy brings to the device pool `pool`."""
@@ -498,9 +531,10 @@ class CtdetDetector:
             H, W = frame.shape
             planes = tuple(pool.data_ptr() + off for off in offsets)
             pitch, kind, step = (W, W // 2), WARP_SRC_YUV420, 1
-        for k, (sh, sw, M, _) in enumerate(layout):
+        H, W = frame.shape[:2]
+        for k, (_, _, M, _) in enumerate(layout):
             slot = slot0 + n * k
-            desc[k] = (planes, pitch, kind, step, sh, sw, np.asarray(M, np.float64).reshape(6), slot, slot + 1 if n == 2 else -1)
+            desc[k] = (planes, pitch, kind, step, H, W, np.asarray(M, np.float64).reshape(6), slot, slot + 1 if n == 2 else -1)
 
     def _slots_u8(self, image, scales, ih, iw):
         """The network images of `scales` of one uint8 HWC frame as one uint8 CUDA batch [slots, ih, iw, 3] (scale-major, the
@@ -641,8 +675,8 @@ class CtdetDetector:
         unquantised model takes the same steps with one cdn_warp_affine_u8_f32_batch launch instead, which writes normalised
         fp32 NCHW slots through the 3 x 256 table run() uses for each scale (_device_table, _norm_tables), then EngineF32
         eagerly (_forward_float).  When
-        the one test scale is 1 and a step holds at least JPEG_DEVICE_MIN_FRAMES frames, the JPEG streams the device takes
-        (cdn_jpeg_parse) go up compressed in the same staging copy,
+        the one test scale is 1 (or with opt.device_resize, below) and a step holds at least JPEG_DEVICE_MIN_FRAMES frames, the
+        JPEG streams the quantised model's device decode takes (cdn_jpeg_parse) go up compressed in the same staging copy,
         with their descriptors, and one cdn_jpeg_decode_batch call decodes them into the device pool the warp reads; other
         encoded inputs are decoded by cv2 on the host first.  Two staging buffers, kept on the detector, let the packing and
         copy of step n + 1 overlap the compute of step n.  After the last step one post-affine, grouping, cdn_ctdet_merge over
@@ -658,7 +692,16 @@ class CtdetDetector:
         the unquantised model, cdn_warp_affine_src_u8_f32_batch) launch: CUDA planes are read in place, with none of their bytes
         staged, host YUV420 planes are staged at 1.5 bytes per pixel and converted to BGR tap by tap inside the warp, and the
         step's host arrays and device-decoded JPEGs are read from the pool as usual.  At other scale lists they take the host
-        path (one device -> host copy per CUDA frame, to_bgr per YUV420 frame, then the host cv2.resize): correct, not fast.
+        path (one device -> host copy per CUDA frame, to_bgr per YUV420 frame, then the host cv2.resize) unless opt.device_resize
+        is set.
+
+        With opt.device_resize (off by default) at a scale list other than [1], the cv2.resize of pre_process runs inside the warp
+        for every frame whose every scale's resize device_resize_exact accepts: host arrays are staged once at 1x, CUDA planes read in place, host YUV420 planes
+        staged at 1.5 bytes per pixel, JPEGs decoded on the device as above, and one cdn_warp_affine_resize_u8_batch (or
+        cdn_warp_affine_resize_u8_f32_batch) launch per step writes every slot, mirrors included.  A frame outside the predicate
+        takes the host path (one device -> host copy per CUDA frame, to_bgr per YUV420 frame, cv2 decoding, then the host
+        cv2.resize per scale) and its copies go into the same pool and the same launch.  Steps with no frame to resize on the
+        device, and every step without opt.device_resize, launch what they launched before.
         CUDA frames are read on the current stream of the detector's device, after the work already queued there: a frame
         produced on another stream must be synchronised with it by the caller.  They may be freed once run_batch returns."""
         from .. import jpeg
@@ -675,7 +718,8 @@ class CtdetDetector:
         layouts = [self._frame_layout(h, w, self.scales) for h, w in shapes]
         metas = [m for layout in layouts for _, _, _, m in layout]
         max_batch = getattr(opt, "max_batch", 1)
-        steps = plan_frame_steps([_staged_sources(items[f], layouts[f]) for f in range(F)], spf, max_batch)
+        resized = [self._resized_on_device(item) for item in items]
+        steps = plan_frame_steps([_staged_sources(items[f], layouts[f], resized[f]) for f in range(F)], spf, max_batch)
         step_slots = max(int(max_batch), spf)
         on_dev = [f for f in range(F) if items[f][1] is not None]
         rank = {f: k for k, f in enumerate(on_dev)}
@@ -709,23 +753,30 @@ class CtdetDetector:
                 wdesc = np.zeros(len(fr) * S, WARP_DESC)
                 for k, f in enumerate(fr):
                     image, data, _ = items[f]
-                    if image is not None:
+                    if image is not None and resized[f]:
+                        # staged once at 1x: the kernel resizes it for every test scale
+                        off = offsets[k][0]
+                        host[off:off + image.size] = np.ascontiguousarray(image).reshape(-1)
+                        self._frame_descs(wdesc[k * S:(k + 1) * S], off, image.shape[:2], layouts[f], k * spf)
+                    elif image is not None:
                         self._pack_frame(image, layouts[f], self.scales, host, offsets[k], wdesc[k * S:(k + 1) * S], k * spf)
                     elif data is not None:
                         j = jf.index(f)
                         host[soffs[j]:soffs[j] + data.size] = data
-                        (sh, sw, M, _), = layouts[f]
-                        wdesc[k] = (desc[j]["out_offset"], sh, sw, np.asarray(M, np.float64).reshape(6), k * spf,
-                                    k * spf + 1 if n == 2 else -1)
+                        self._frame_descs(wdesc[k * S:(k + 1) * S], desc[j]["out_offset"], shapes[f], layouts[f], k * spf)
                 if jf:
                     host[table:table + desc.nbytes] = desc.view(np.uint8)
                 sdesc = None
-                if direct:
+                resize = any(resized[f] for f in fr)
+                if direct or resize:
                     # one general-source launch writes every slot of the step: the pool's frames as pitched BGR descriptors
                     sdesc = _pool_src_descs(wdesc, pool)
                     for k in direct:
                         f = fr[k]
                         self._frame_src_descs(items[f][2], layouts[f], host, pool, offsets[k], sdesc[k * S:(k + 1) * S], k * spf)
+                if resize:
+                    # every descriptor's frame resized to its scale's size inside the warp (the host-resized copies at 1:1)
+                    sdesc = _rs_descs(sdesc, [(sh, sw) for f in fr for sh, sw, _, _ in layouts[f]])
                 if staged:
                     if grown:
                         # a new pool may reuse memory the compute stream freed with work still queued (e.g. the flip merge's maps)
@@ -744,11 +795,11 @@ class CtdetDetector:
                                       pool.data_ptr(), pool.numel(), status[rank[jf[0]]:].data_ptr(), compute.cuda_stream)
                 if self.float_model:
                     table_index = self._table_index(self.scales, len(fr))
-                    if direct:
+                    if direct or resize:
                         self._warp_src_f32(sdesc, table_index, st["tables"], st["dst"])
                     else:
                         self._warp_f32(pool, wdesc, table_index, st["tables"], st["dst"])
-                elif direct:
+                elif direct or resize:
                     self._warp_src(sdesc, st["dst"])
                 else:
                     self._warp(pool, wdesc, st["dst"])
@@ -777,9 +828,9 @@ class CtdetDetector:
     def _batch_frames(self, frames):
         """run_batch's inputs checked and loaded -> [(image, encoded bytes, JPEG descriptor)]: uint8 HWC 3-channel arrays as
         they are (image, None, None); paths (read as bytes) and encoded images as (None, bytes, descriptor) when the device
-        decodes them (the quantised model, test_scales == [1], at least JPEG_DEVICE_MIN_FRAMES frames per engine step,
-        cdn_jpeg_parse accepts the stream), else decoded by cv2.imdecode, which is what cv2.imread does after reading the file
-        (image, None, None)."""
+        decodes them (the quantised model, test_scales == [1] or _device_resize with _resize_exact accepting the frame's size, at
+        least JPEG_DEVICE_MIN_FRAMES frames per engine step, cdn_jpeg_parse accepts the stream), else decoded by cv2.imdecode,
+        which is what cv2.imread does after reading the file (image, None, None)."""
         from .. import jpeg
         if not self.opt.fix_res:
             raise ValueError("run_batch needs fix_res: without it every input size compiles its own engine; use run() for keep_res")
@@ -800,18 +851,20 @@ class CtdetDetector:
         # (13-41 ms for 500x375 q75-q95 on a B200) whatever the number of frames: it pays from JPEG_DEVICE_MIN_FRAMES per step
         spf = len(self.opt.test_scales) * (2 if self.opt.flip_test else 1)
         per_step = max(int(getattr(self.opt, "max_batch", 1)), spf) // spf
-        device_jpeg = (self.opt.resume_quantize and list(self.opt.test_scales) == [1] and
-                       min(per_step, len(frames)) >= JPEG_DEVICE_MIN_FRAMES)
-        # CUDA and YUV420 frames go to the general-source warp when every test scale is 1; otherwise pre_process's host cv2.resize
-        # needs them as host BGR images (one device -> host copy per CUDA frame, to_bgr per YUV420 frame): correct, not fast
+        # CUDA, YUV420 and device-decoded frames stay on the device when every test scale is 1, or with _device_resize when the
+        # device resize reproduces every scale's cv2.resize of them (_resize_exact); otherwise pre_process's host cv2.resize needs
+        # them as host BGR images (one device -> host copy per CUDA frame, to_bgr per YUV420 frame, cv2 decoding)
         direct = all(s == 1 for s in self.opt.test_scales)
+        resize = self._device_resize()
+        device_jpeg = (self.opt.resume_quantize and (list(self.opt.test_scales) == [1] or resize) and
+                       min(per_step, len(frames)) >= JPEG_DEVICE_MIN_FRAMES)
         items = []
         for f in frames:
             if isinstance(f, np.ndarray) and f.ndim == 3:
                 items.append((f, None, None))
                 continue
             if _is_frame(f):
-                items.append((None, None, f) if direct else
+                items.append((None, None, f) if direct or (resize and self._resize_exact(*f.shape[:2])) else
                              (f.cpu().numpy() if isinstance(f, torch.Tensor) else to_bgr(f), None, None))
                 continue
             if isinstance(f, str):
@@ -824,7 +877,7 @@ class CtdetDetector:
                 data = jpeg.as_bytes(f)
             if device_jpeg:
                 rc, desc = jpeg.parse(data)
-                if rc == 0:
+                if rc == 0 and (not resize or self._resize_exact(int(desc[0]["height"]), int(desc[0]["width"]))):
                     items.append((None, data, desc))
                     continue
             try:
@@ -908,13 +961,14 @@ def _item_shape(item):
     return tuple(int(v) for v in x.shape[:2])
 
 
-def _staged_sources(item, layout):
+def _staged_sources(item, layout, resized=False):
     """The byte sizes of what run_batch stages for one _batch_frames item (plan_frame_steps' source_bytes): the source image of
-    every test scale of a host array, the Y, U and V planes of a host YUV420 frame; nothing for a CUDA frame, read in place, or a
-    device-decoded JPEG, whose stream is staged after the raw sources of its step."""
+    every test scale of a host array (the array once when the device resizes it, `resized`), the Y, U and V planes of a host
+    YUV420 frame; nothing for a CUDA frame, read in place, or a device-decoded JPEG, whose stream is staged after the raw sources
+    of its step."""
     image, _, x = item
     if image is not None:
-        return [sh * sw * 3 for sh, sw, _, _ in layout]
+        return [image.size] if resized else [sh * sw * 3 for sh, sw, _, _ in layout]
     if isinstance(x, YUV420) and not x.is_cuda:
         H, W = x.shape
         return [H * W, H * W // 4, H * W // 4]
@@ -931,11 +985,36 @@ def _pool_src_descs(wdesc, pool):
     for k in ("src_h", "src_w", "M", "dst_slot", "mirror_slot"):
         d[k] = wdesc[k]
     return d
+def _rs_descs(sdesc, resized):
+    """General-source descriptors (_lib.WARP_SRC_DESC, source size the frame's) -> resize descriptors (_lib.WARP_RS_DESC): entry i
+    resizes its frame to resized[i] = (height, width), the identity where that is the frame's size."""
+    from .._lib import WARP_RS_DESC
+    d = np.zeros(len(sdesc), WARP_RS_DESC)
+    for k in ("plane", "pitch", "kind", "chroma_step", "src_h", "src_w", "M", "dst_slot", "mirror_slot"):
+        d[k] = sdesc[k]
+    rs = np.asarray(resized, np.int32).reshape(-1, 2)
+    d["rs_h"], d["rs_w"] = rs[:, 0], rs[:, 1]
+    # the expressions cdn_warp_affine_resize_* checks, in float64 like OpenCV's 1 / inv_scale
+    d["inv_scale"][:, 0] = 1.0 / (d["rs_w"].astype(np.float64) / d["src_w"])
+    d["inv_scale"][:, 1] = 1.0 / (d["rs_h"].astype(np.float64) / d["src_h"])
+    return d
+
+
 MERGE_MAX_ROWS = 1024          # CDN_SOFT_NMS_MAX_LEN: test scales x K rows per image that cdn_ctdet_merge takes
 # frames per run_batch step from which JPEGs are decoded on the device rather than by cv2 on the host: on one B200 (1000 W) with
 # 500x375 4:2:0 files the device decode lost at 16 frames per step and at 32 frames at q95, and won from 64 frames per step
 # (profiles/r04_jpeg_decode.json, run_batch rows "paths_device_decode" against "host_imread_then_arrays")
 JPEG_DEVICE_MIN_FRAMES = 48
+RESIZE_MAX_SIDE = 4096         # the largest frame and resized side device_resize_exact accepts
+
+
+def device_resize_exact(H, W, sh, sw):
+    """True when cdn_warp_affine_resize_u8[_f32]_batch's resize is cv2.resize(frame, (sw, sh)) of an H x W frame bit for bit: the
+    geometry tests/test_resize_cpu.py pins against cv2 (oracle.resize_ref restates the rule, DESIGN.md section 9).  Every side
+    from 1 to RESIZE_MAX_SIDE, each resized side between a fifth of the frame's side and three times it.  run_batch resizes other
+    frames with cv2 on the host."""
+    return (all(1 <= int(v) <= RESIZE_MAX_SIDE for v in (H, W, sh, sw)) and
+            5 * sh >= H and 5 * sw >= W and sh <= 3 * H and sw <= 3 * W)
 
 
 def plan_scale_batches(sizes):

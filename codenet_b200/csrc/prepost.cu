@@ -57,6 +57,21 @@ struct WarpSrcF32Params {
   WarpSrcDesc d[WARP_SRC_F32_MAX_DESC]; uint8_t table[WARP_SRC_F32_MAX_DESC];
 };
 static_assert(offsetof(WarpSrcF32Params, d) == 32 && sizeof(WarpSrcF32Params) <= 32764, "WarpSrcF32Params");
+// cdn_warp_rs_desc on the device: the warp sees an H x W image (the resized size), read from an FH x FW frame
+struct WarpRsDesc { const uint8_t* p[3]; long long pitch[2]; double m[6]; double scale[2]; int H, W, FH, FW, kind, step, dst, mirror; };
+static_assert(sizeof(WarpRsDesc) == 136, "WarpRsDesc layout");
+static_assert(sizeof(cdn_warp_rs_desc) == 136, "cdn_warp_rs_desc layout (codenet_b200._lib.WARP_RS_DESC)");
+constexpr int WARP_RS_MAX_DESC = (32764 - 24) / (int)sizeof(WarpRsDesc);
+static_assert(WARP_RS_MAX_DESC == CDN_WARP_RS_DESC_PER_LAUNCH, "include/codenet_b200.h states the descriptors per launch");
+struct WarpRsParams { uint8_t* dst; int dh, dw, groups, pad; WarpRsDesc d[WARP_RS_MAX_DESC]; };
+static_assert(offsetof(WarpRsParams, d) == 24 && sizeof(WarpRsParams) <= 32764, "WarpRsParams");
+constexpr int WARP_RS_F32_MAX_DESC = (32764 - 32) / (int)(sizeof(WarpRsDesc) + sizeof(uint8_t));
+static_assert(WARP_RS_F32_MAX_DESC == CDN_WARP_RS_F32_DESC_PER_LAUNCH, "include/codenet_b200.h states the descriptors per launch");
+struct WarpRsF32Params {
+  float* dst; const float* tables; int dh, dw, groups, vec;
+  WarpRsDesc d[WARP_RS_F32_MAX_DESC]; uint8_t table[WARP_RS_F32_MAX_DESC];
+};
+static_assert(offsetof(WarpRsF32Params, d) == 32 && sizeof(WarpRsF32Params) <= 32764, "WarpRsF32Params");
 
 // cv::warpAffine's inversion of the 2 x 3 matrix (imgwarp.cpp), in double on the host: the same expressions on the device
 // would be contracted into FMAs and could round differently
@@ -115,6 +130,45 @@ struct Yuv420 {
     acc[0] += min(max((l + YUV_CUB * U) >> YUV_SHIFT, 0), 255) * w;
     acc[1] += min(max((l + YUV_CVG * V + YUV_CUG * U) >> YUV_SHIFT, 0), 255) * w;
     acc[2] += min(max((l + YUV_CVR * V) >> YUV_SHIFT, 0), 255) * w;
+  }
+};
+
+// cv2.resize's INTER_LINEAR coefficients of destination index d for 8-bit images (resize.cpp): the two source indices s0, s1
+// (clipped into [0, n)) and their 11-bit weights c0, c1.  fx = float((d + 0.5) * scale - 0.5) in OpenCV's rounding order (the
+// intrinsics keep nvcc from contracting into FMAs), floor, the fraction, then saturate_cast<short>, which rounds half to even.
+// Columns (clamp) left of the frame or past its last pixel take that pixel at full weight; rows keep their fraction even there,
+// so an upscale's first and last rows read one row twice with two truncating products (DESIGN.md section 9).
+__device__ __forceinline__ void resize_coef(int d, double scale, int n, bool clamp, int& s0, int& s1, int& c0, int& c1) {
+  float f = __double2float_rn(__dadd_rn(__dmul_rn(__dadd_rn((double)d, 0.5), scale), -0.5));
+  const float fl = floorf(f);
+  int s = (int)fl;
+  f = __fsub_rn(f, fl);
+  if (clamp && (s < 0 || s >= n - 1)) {
+    s = min(max(s, 0), n - 1);
+    f = 0.f;
+  }
+  c0 = __float2int_rn(__fmul_rn(__fsub_rn(1.f, f), 2048.f));
+  c1 = __float2int_rn(__fmul_rn(f, 2048.f));
+  s0 = min(max(s, 0), n - 1);
+  s1 = min(max(s + 1, 0), n - 1);
+}
+
+// A tap of the resized image: pixel (yy, xx) of cv2.resize(frame, (rs_w, rs_h)) from four frame pixels read by Src, with
+// OpenCV's passes: exact horizontal sums S = p0 * a0 + p1 * a1 (< 2^20), then (((b0 * (S0 >> 4)) >> 16) + ((b1 * (S1 >> 4)) >>
+// 16) + 2) >> 2 (every product < 2^27).  Each frame pixel goes through Src as it is, so a YUV frame is converted before it is
+// resized, as cv2.resize(cv2.cvtColor(frame, ...)) sees it.
+template <class Src>
+struct Resized {
+  Src src; int H, W; double sx, sy;                  // the frame's size; 1 / (rs_w / W), 1 / (rs_h / H)
+  __device__ __forceinline__ void operator()(int yy, int xx, int w, int (&acc)[3]) const {
+    int x0, x1, a0, a1, y0, y1, b0, b1;
+    resize_coef(xx, sx, W, true, x0, x1, a0, a1);
+    resize_coef(yy, sy, H, false, y0, y1, b0, b1);
+    int s0[3] = {0, 0, 0}, s1[3] = {0, 0, 0};
+    src(y0, x0, a0, s0); src(y0, x1, a1, s0);
+    src(y1, x0, a0, s1); src(y1, x1, a1, s1);
+#pragma unroll
+    for (int c = 0; c < 3; ++c) acc[c] += min((((b0 * (s0[c] >> 4)) >> 16) + ((b1 * (s1[c] >> 4)) >> 16) + 2) >> 2, 255) * w;
   }
 };
 
@@ -284,6 +338,85 @@ __global__ void __launch_bounds__(WARP_THREADS) warp_affine_src_u8_f32_kernel(co
   }
 }
 
+// The resize-and-warp kernels: the general-source kernels with every tap of the warp a pixel of the resized frame (Resized), or
+// of the frame itself where the descriptor's resized size is the frame's (the branch is uniform per CTA).
+template <class Src>
+__device__ __forceinline__ void warp_rs_pixels_of(const WarpRsDesc& q, const Src& src, int y, int x0, uint8_t (&v)[WARP_PX * 3]) {
+  if (q.FH == q.H && q.FW == q.W)
+    warp_pixels(q, src, y, x0, v);
+  else
+    warp_pixels(q, Resized<Src>{src, q.FH, q.FW, q.scale[0], q.scale[1]}, y, x0, v);
+}
+
+__device__ __forceinline__ void warp_rs_pixels(const WarpRsDesc& q, int y, int x0, uint8_t (&v)[WARP_PX * 3]) {
+  if (q.kind == CDN_WARP_SRC_YUV420)
+    warp_rs_pixels_of(q, Yuv420{q.p[0], q.p[1], q.p[2], q.pitch[0], q.pitch[1], q.step}, y, x0, v);
+  else
+    warp_rs_pixels_of(q, PitchedBgr{q.p[0], q.pitch[0]}, y, x0, v);
+}
+
+__global__ void __launch_bounds__(WARP_THREADS) warp_affine_resize_u8_kernel(const __grid_constant__ WarpRsParams p) {
+  const WarpRsDesc& q = p.d[blockIdx.y];
+  const int t = blockIdx.x * WARP_THREADS + threadIdx.x;
+  const int y = t / p.groups, x0 = (t - y * p.groups) * WARP_PX;
+  if (y >= p.dh) return;
+  const int n = min(WARP_PX, p.dw - x0);
+  uint8_t v[WARP_PX * 3];
+  warp_rs_pixels(q, y, x0, v);
+  const size_t plane = (size_t)p.dh * p.dw * 3, row = (size_t)y * p.dw * 3;
+  warp_store(p.dst + (size_t)q.dst * plane + row + (size_t)x0 * 3, v, n);
+  if (q.mirror >= 0) {
+    uint8_t f[WARP_PX * 3];
+#pragma unroll
+    for (int i = 0; i < WARP_PX; ++i)
+#pragma unroll
+      for (int c = 0; c < 3; ++c) f[i * 3 + c] = v[(WARP_PX - 1 - i) * 3 + c];
+    uint8_t* m = p.dst + (size_t)q.mirror * plane + row + (size_t)(p.dw - x0 - n) * 3;
+    if (n == WARP_PX) {
+      warp_store(m, f, n);
+    } else {
+      const int skip = (WARP_PX - n) * 3;
+#pragma unroll
+      for (int i = 0; i < WARP_PX * 3; ++i)
+        if (i >= skip) m[i - skip] = f[i];
+    }
+  }
+}
+
+__global__ void __launch_bounds__(WARP_THREADS) warp_affine_resize_u8_f32_kernel(const __grid_constant__ WarpRsF32Params p) {
+  __shared__ float s_tab[3 * 256];
+  const WarpRsDesc& q = p.d[blockIdx.y];
+  const float* tab = p.tables + (size_t)p.table[blockIdx.y] * (3 * 256);
+  for (int i = threadIdx.x; i < 3 * 256; i += WARP_THREADS) s_tab[i] = __ldg(tab + i);
+  __syncthreads();
+  const int t = blockIdx.x * WARP_THREADS + threadIdx.x;
+  const int y = t / p.groups, x0 = (t - y * p.groups) * WARP_PX;
+  if (y >= p.dh) return;
+  const int n = min(WARP_PX, p.dw - x0);
+  uint8_t v[WARP_PX * 3];
+  warp_rs_pixels(q, y, x0, v);
+  const size_t plane = (size_t)p.dh * p.dw, row = (size_t)y * p.dw;
+  float* d = p.dst + (size_t)q.dst * 3 * plane + row + x0;
+  float* m = q.mirror >= 0 ? p.dst + (size_t)q.mirror * 3 * plane + row + (p.dw - x0 - n) : nullptr;
+#pragma unroll
+  for (int c = 0; c < 3; ++c) {
+    float f[WARP_PX];
+#pragma unroll
+    for (int i = 0; i < WARP_PX; ++i) f[i] = s_tab[c * 256 + v[i * 3 + c]];
+    if (p.vec) {
+      *reinterpret_cast<float4*>(d + c * plane) = make_float4(f[0], f[1], f[2], f[3]);
+      if (m) *reinterpret_cast<float4*>(m + c * plane) = make_float4(f[3], f[2], f[1], f[0]);
+    } else {
+#pragma unroll
+      for (int i = 0; i < WARP_PX; ++i)
+        if (i < n) {
+          d[c * plane + i] = f[i];
+          if (m) m[c * plane + n - 1 - i] = f[i];
+        }
+    }
+  }
+}
+
 // the destination checks of every batch entry point
 static int warp_dst_check(const char* who, int n, int dst_slots, int dst_h, int dst_w) {
   CDN_CHECK(n >= 0, CDN_ERR_INVALID, "%s: n = %d", who, n);
@@ -309,31 +442,50 @@ static int warp_batch_check(const char* who, const cdn_warp_desc* h_desc, int n,
   return 0;
 }
 
-// the checks both general-source entry points make before anything is launched: what every plane must hold, per source kind
+// the checks the general-source and the resize entry points make on a descriptor before anything is launched: what every plane
+// must hold, per source kind
+template <class Desc>
+static int warp_frame_check(const char* who, const Desc& d, int i, int dst_slots) {
+  CDN_CHECK(d.kind == CDN_WARP_SRC_BGR || d.kind == CDN_WARP_SRC_YUV420, CDN_ERR_INVALID, "%s: descriptor %d: unknown source kind %d",
+          who, i, d.kind);
+  CDN_CHECK(d.src_h > 0 && d.src_w > 0, CDN_ERR_INVALID, "%s: descriptor %d: bad source size %d x %d", who, i, d.src_h, d.src_w);
+  if (d.kind == CDN_WARP_SRC_BGR) {
+    CDN_CHECK(d.plane[0], CDN_ERR_INVALID, "%s: descriptor %d: null plane", who, i);
+    CDN_CHECK(d.pitch[0] >= 3LL * d.src_w, CDN_ERR_INVALID, "%s: descriptor %d: pitch %lld below the row's %lld bytes", who, i,
+              d.pitch[0], 3LL * d.src_w);
+  } else {
+    CDN_CHECK(d.plane[0] && d.plane[1] && d.plane[2], CDN_ERR_INVALID, "%s: descriptor %d: null plane", who, i);
+    CDN_CHECK(d.src_h % 2 == 0 && d.src_w % 2 == 0, CDN_ERR_INVALID, "%s: descriptor %d: odd YUV 4:2:0 size %d x %d", who, i,
+              d.src_h, d.src_w);
+    CDN_CHECK(d.chroma_step == 1 || d.chroma_step == 2, CDN_ERR_INVALID, "%s: descriptor %d: chroma step %d not 1 or 2", who, i,
+              d.chroma_step);
+    const long long chroma_row = (long long)(d.src_w / 2 - 1) * d.chroma_step + 1;
+    CDN_CHECK(d.pitch[0] >= d.src_w && d.pitch[1] >= chroma_row, CDN_ERR_INVALID,
+              "%s: descriptor %d: pitch %lld / %lld below the rows' %d / %lld bytes", who, i, d.pitch[0], d.pitch[1], d.src_w,
+              chroma_row);
+  }
+  CDN_CHECK(d.dst_slot >= 0 && d.dst_slot < dst_slots && d.mirror_slot >= -1 && d.mirror_slot < dst_slots, CDN_ERR_INVALID,
+            "%s: descriptor %d: slot %d / mirror %d outside [0, %d)", who, i, d.dst_slot, d.mirror_slot, dst_slots);
+  return 0;
+}
+
 static int warp_src_check(const char* who, const cdn_warp_src_desc* h_desc, int n, int dst_slots, int dst_h, int dst_w) {
   if (int rc = warp_dst_check(who, n, dst_slots, dst_h, dst_w)) return rc;
+  for (int i = 0; i < n; ++i)
+    if (int rc = warp_frame_check(who, h_desc[i], i, dst_slots)) return rc;
+  return 0;
+}
+
+// the resize entry points: the frame checks plus a resized size of at least 1 x 1 whose scales are the descriptor's, bit for bit
+static int warp_rs_check(const char* who, const cdn_warp_rs_desc* h_desc, int n, int dst_slots, int dst_h, int dst_w) {
+  if (int rc = warp_dst_check(who, n, dst_slots, dst_h, dst_w)) return rc;
   for (int i = 0; i < n; ++i) {
-    const cdn_warp_src_desc& d = h_desc[i];
-    CDN_CHECK(d.kind == CDN_WARP_SRC_BGR || d.kind == CDN_WARP_SRC_YUV420, CDN_ERR_INVALID, "%s: descriptor %d: unknown source kind %d",
-              who, i, d.kind);
-    CDN_CHECK(d.src_h > 0 && d.src_w > 0, CDN_ERR_INVALID, "%s: descriptor %d: bad source size %d x %d", who, i, d.src_h, d.src_w);
-    if (d.kind == CDN_WARP_SRC_BGR) {
-      CDN_CHECK(d.plane[0], CDN_ERR_INVALID, "%s: descriptor %d: null plane", who, i);
-      CDN_CHECK(d.pitch[0] >= 3LL * d.src_w, CDN_ERR_INVALID, "%s: descriptor %d: pitch %lld below the row's %lld bytes", who, i,
-                d.pitch[0], 3LL * d.src_w);
-    } else {
-      CDN_CHECK(d.plane[0] && d.plane[1] && d.plane[2], CDN_ERR_INVALID, "%s: descriptor %d: null plane", who, i);
-      CDN_CHECK(d.src_h % 2 == 0 && d.src_w % 2 == 0, CDN_ERR_INVALID, "%s: descriptor %d: odd YUV 4:2:0 size %d x %d", who, i,
-                d.src_h, d.src_w);
-      CDN_CHECK(d.chroma_step == 1 || d.chroma_step == 2, CDN_ERR_INVALID, "%s: descriptor %d: chroma step %d not 1 or 2", who, i,
-                d.chroma_step);
-      const long long chroma_row = (long long)(d.src_w / 2 - 1) * d.chroma_step + 1;
-      CDN_CHECK(d.pitch[0] >= d.src_w && d.pitch[1] >= chroma_row, CDN_ERR_INVALID,
-                "%s: descriptor %d: pitch %lld / %lld below the rows' %d / %lld bytes", who, i, d.pitch[0], d.pitch[1], d.src_w,
-                chroma_row);
-    }
-    CDN_CHECK(d.dst_slot >= 0 && d.dst_slot < dst_slots && d.mirror_slot >= -1 && d.mirror_slot < dst_slots, CDN_ERR_INVALID,
-              "%s: descriptor %d: slot %d / mirror %d outside [0, %d)", who, i, d.dst_slot, d.mirror_slot, dst_slots);
+    const cdn_warp_rs_desc& d = h_desc[i];
+    if (int rc = warp_frame_check(who, d, i, dst_slots)) return rc;
+    CDN_CHECK(d.rs_h > 0 && d.rs_w > 0, CDN_ERR_INVALID, "%s: descriptor %d: bad resized size %d x %d", who, i, d.rs_h, d.rs_w);
+    CDN_CHECK(d.inv_scale[0] == 1. / ((double)d.rs_w / d.src_w) && d.inv_scale[1] == 1. / ((double)d.rs_h / d.src_h), CDN_ERR_INVALID,
+              "%s: descriptor %d: scales %.17g, %.17g are not those of %d x %d -> %d x %d", who, i, d.inv_scale[0], d.inv_scale[1],
+              d.src_h, d.src_w, d.rs_h, d.rs_w);
   }
   return 0;
 }
@@ -435,6 +587,60 @@ extern "C" int cdn_warp_affine_src_u8_f32_batch(const cdn_warp_src_desc* h_desc,
     }
     warp_affine_src_u8_f32_kernel<<<dim3((unsigned)tiles, (unsigned)m), WARP_THREADS, 0, (cudaStream_t)stream>>>(p);
     CDN_LAUNCH_CHECK("warp_affine_src_u8_f32_kernel");
+  }
+  return 0;
+}
+
+static void warp_rs_fill(const cdn_warp_rs_desc& d, WarpRsDesc& q) {
+  for (int k = 0; k < 3; ++k) q.p[k] = d.plane[k];
+  q.pitch[0] = d.pitch[0]; q.pitch[1] = d.pitch[1];
+  q.scale[0] = d.inv_scale[0]; q.scale[1] = d.inv_scale[1];
+  q.H = d.rs_h; q.W = d.rs_w; q.FH = d.src_h; q.FW = d.src_w;
+  q.kind = d.kind; q.step = d.chroma_step; q.dst = d.dst_slot; q.mirror = d.mirror_slot;
+  warp_invert(d.M, q.m);
+}
+
+extern "C" int cdn_warp_affine_resize_u8_batch(const cdn_warp_rs_desc* h_desc, int n, uint8_t* d_dst, int dst_slots, int dst_h,
+                                               int dst_w, cdn_stream_t stream) {
+  CDN_CHECK(h_desc && d_dst, CDN_ERR_INVALID, "warp_affine_resize_batch: null pointer");
+  if (int rc = warp_rs_check("warp_affine_resize_batch", h_desc, n, dst_slots, dst_h, dst_w)) return rc;
+  const int groups = (dst_w + WARP_PX - 1) / WARP_PX;
+  const long long tiles = ((long long)dst_h * groups + WARP_THREADS - 1) / WARP_THREADS;
+  WarpRsParams p;
+  p.dst = d_dst; p.dh = dst_h; p.dw = dst_w; p.groups = groups; p.pad = 0;
+  for (int base = 0; base < n; base += WARP_RS_MAX_DESC) {
+    const int m = std::min(WARP_RS_MAX_DESC, n - base);
+    for (int i = 0; i < m; ++i) warp_rs_fill(h_desc[base + i], p.d[i]);
+    warp_affine_resize_u8_kernel<<<dim3((unsigned)tiles, (unsigned)m), WARP_THREADS, 0, (cudaStream_t)stream>>>(p);
+    CDN_LAUNCH_CHECK("warp_affine_resize_u8_kernel");
+  }
+  return 0;
+}
+
+extern "C" int cdn_warp_affine_resize_u8_f32_batch(const cdn_warp_rs_desc* h_desc, const int32_t* h_table, int n,
+                                                   const float* d_tables, int n_tables, float* d_dst, int dst_slots, int dst_h,
+                                                   int dst_w, cdn_stream_t stream) {
+  CDN_CHECK(h_desc && h_table && d_tables && d_dst, CDN_ERR_INVALID, "warp_affine_resize_f32_batch: null pointer");
+  CDN_CHECK(((uintptr_t)d_tables & 3) == 0 && ((uintptr_t)d_dst & 3) == 0, CDN_ERR_INVALID,
+            "warp_affine_resize_f32_batch: tables and destination must be 4-byte aligned");
+  CDN_CHECK(n_tables >= 1 && n_tables <= 2, CDN_ERR_INVALID, "warp_affine_resize_f32_batch: n_tables = %d outside [1, 2]", n_tables);
+  if (int rc = warp_rs_check("warp_affine_resize_f32_batch", h_desc, n, dst_slots, dst_h, dst_w)) return rc;
+  for (int i = 0; i < n; ++i)
+    CDN_CHECK(h_table[i] >= 0 && h_table[i] < n_tables, CDN_ERR_INVALID,
+              "warp_affine_resize_f32_batch: descriptor %d: table %d outside [0, %d)", i, h_table[i], n_tables);
+  const int groups = (dst_w + WARP_PX - 1) / WARP_PX;
+  const long long tiles = ((long long)dst_h * groups + WARP_THREADS - 1) / WARP_THREADS;
+  WarpRsF32Params p;
+  p.dst = d_dst; p.tables = d_tables; p.dh = dst_h; p.dw = dst_w; p.groups = groups;
+  p.vec = dst_w % WARP_PX == 0 && ((uintptr_t)d_dst & 15) == 0;
+  for (int base = 0; base < n; base += WARP_RS_F32_MAX_DESC) {
+    const int m = std::min(WARP_RS_F32_MAX_DESC, n - base);
+    for (int i = 0; i < m; ++i) {
+      warp_rs_fill(h_desc[base + i], p.d[i]);
+      p.table[i] = (uint8_t)h_table[base + i];
+    }
+    warp_affine_resize_u8_f32_kernel<<<dim3((unsigned)tiles, (unsigned)m), WARP_THREADS, 0, (cudaStream_t)stream>>>(p);
+    CDN_LAUNCH_CHECK("warp_affine_resize_u8_f32_kernel");
   }
   return 0;
 }

@@ -194,6 +194,34 @@ int cdn_warp_affine_src_u8_batch(const cdn_warp_src_desc* h_desc, int n, uint8_t
                                  cdn_stream_t stream);
 int cdn_warp_affine_src_u8_f32_batch(const cdn_warp_src_desc* h_desc, const int32_t* h_table, int n, const float* d_tables,
                                      int n_tables, float* d_dst, int dst_slots, int dst_h, int dst_w, cdn_stream_t stream);
+
+/* cdn_warp_affine_resize_u8_batch / cdn_warp_affine_resize_u8_f32_batch: cdn_warp_affine_src_u8[_f32]_batch with the cv2.resize of
+ * BaseDetector.pre_process in front of the warp.  Each cdn_warp_rs_desc holds a src_h x src_w frame (plane, pitch, kind and
+ * chroma_step as in cdn_warp_src_desc) and the size rs_h x rs_w it is resized to; M maps the RESIZED image to the network input.
+ * Output slot dst_slot is cv2.warpAffine(cv2.resize(frame, (rs_w, rs_h)), M, (dst_w, dst_h), flags=cv2.INTER_LINEAR) bit for bit
+ * (YUV frames: of cv2.cvtColor(frame, COLOR_YUV2BGR_*)), for the geometry codenet_b200.compat.detector.device_resize_exact accepts:
+ * every tap of the warp is a resized pixel computed from four frame pixels with OpenCV's 11-bit fixed-point INTER_LINEAR
+ * arithmetic (DESIGN.md section 9).  rs_h == src_h and rs_w == src_w reads the frame as it is.  inv_scale holds 1 / (rs_w / src_w)
+ * and 1 / (rs_h / src_h) in double, the expressions OpenCV computes its coefficients from.  The checks of
+ * cdn_warp_affine_src_u8[_f32]_batch, plus rs_h, rs_w >= 1 and inv_scale equal to those expressions, all on the host before
+ * anything is launched.  No workspace, allocation or synchronisation.  Up to CDN_WARP_RS[_F32]_DESC_PER_LAUNCH descriptors per
+ * launch. */
+typedef struct cdn_warp_rs_desc {
+  const uint8_t* plane[3];           /* device addresses: BGR plane[0]; YUV Y, U, V */
+  long long pitch[2];                /* row pitch in bytes of plane 0 and of the chroma planes */
+  int kind, chroma_step;             /* CDN_WARP_SRC_*; bytes between chroma samples of a row (1 or 2) */
+  int src_h, src_w;                  /* the frame */
+  int rs_h, rs_w;                    /* the resized image M refers to */
+  double inv_scale[2];               /* 1 / (rs_w / src_w), 1 / (rs_h / src_h) */
+  double M[6];                       /* the 2x3 resized-image -> destination matrix cv2.warpAffine receives, row major */
+  int dst_slot, mirror_slot;
+} cdn_warp_rs_desc;
+#define CDN_WARP_RS_DESC_PER_LAUNCH 240
+#define CDN_WARP_RS_F32_DESC_PER_LAUNCH 238
+int cdn_warp_affine_resize_u8_batch(const cdn_warp_rs_desc* h_desc, int n, uint8_t* d_dst, int dst_slots, int dst_h, int dst_w,
+                                    cdn_stream_t stream);
+int cdn_warp_affine_resize_u8_f32_batch(const cdn_warp_rs_desc* h_desc, const int32_t* h_table, int n, const float* d_tables,
+                                        int n_tables, float* d_dst, int dst_slots, int dst_h, int dst_w, cdn_stream_t stream);
 int cdn_ctdet_group_by_class(const float* d_dets, int batch, int K, int num_classes, float* d_out, int32_t* d_counts,
                              cdn_stream_t stream);
 
